@@ -31,8 +31,6 @@
 // variant 1 (vgsim_set_tau_variant) expands every group, i.e. draws each channel separately exactly like
 // the reference; it is kept as a parity tap.  The same channel code backs the deterministic propensity
 // tap (propensity_kernel).
-#include <stdio.h>
-#include <stdlib.h>
 #include "common.cuh"
 #include "rates.cuh"
 #include "samplers.cuh"
@@ -720,21 +718,14 @@ __device__ __forceinline__ DrawGeom draw_geom(const Dims &D) {
     return g;
 }
 
-#ifndef TAU_THETA
 // a mutation / out-migration group is drawn as ONE Poisson total when lam_total <= theta (exact for any theta < 10).
 // The total wins when it is almost surely 0 (one early-out instead of 9 / 27 channel draws); a non-zero total costs a
 // serial multinomial split in one lane while the warp waits.  Measured at T3: theta 8 / 3 / 1 / 0.3 / 0.15 / 0.1 / 0.03
 // -> 8.60 / 7.19 / 6.38 / 6.17 / 6.16 / 6.19 / 6.43 ms per 131,072 leaps.
-#define TAU_THETA 0.25
-#endif
-// separate thresholds for the two kinds of groups (3U mutation channels / (K-1)S out-migration channels); both < 10
-#ifndef TAU_THETA_MUT
-#define TAU_THETA_MUT TAU_THETA
-#endif
-#ifndef TAU_THETA_MIG
+// Separate thresholds for the two kinds of groups (3U mutation channels / (K-1)S out-migration channels); both < 10.
+#define TAU_THETA_MUT 0.25
 #define TAU_THETA_MIG 0.5  // with the two-stage split of a non-zero total (S + K - 1 terms per event) the (K-1)S out-migration
                            // channels are worth aggregating up to lambda = 0.5: t = 90 12.3 -> 11.8 ms, t = 60 / 120 unchanged
-#endif
 static_assert(TAU_THETA_MUT < 10.0 && TAU_THETA_MIG < 10.0, "aggregated totals are drawn by inversion (lambda < 10)");
 
 // total out-migration propensity of cell (p,h): the sum over targets t and groups s of the channel propensities
@@ -1274,8 +1265,7 @@ namespace vg {
 
 // host launchers ---------------------------------------------------------------------------------
 template <int TEAMS>
-static cudaError_t launch_tau_cfg(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant,
-                                  int ctas_cap) {
+static cudaError_t launch_tau_cfg(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant) {
     const TauShared lay = tau_layout(st.D, false, TAU_TEAM);
     const size_t stride = ((size_t)lay.bytes + 15) & ~(size_t)15;
     const size_t smem = stride * TEAMS + TAU_CTA_TAIL;
@@ -1285,7 +1275,6 @@ static cudaError_t launch_tau_cfg(const DevState &st, const SimArgs &a, cudaStre
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tau_kernel<TEAMS>, TAU_TEAM * TEAMS, smem);
     if (e != cudaSuccess) return e;
     if (per_sm < 1) per_sm = 1;
-    if (ctas_cap > 0 && per_sm > ctas_cap) per_sm = ctas_cap;
     int grid = num_sms * per_sm;
     const int need = (st.R + TEAMS - 1) / TEAMS;
     if (grid > need) grid = need;
@@ -1295,40 +1284,24 @@ static cudaError_t launch_tau_cfg(const DevState &st, const SimArgs &a, cudaStre
 
 // Default: the warp-per-replicate kernel (tau_warp.cuh), one CTA per SM with as many warps as the shared memory
 // holds (<= 14).  The team kernel (256-thread teams, CTA-wide generations) stays available as a parity tap:
-// variant bit 2 (vgsim_set_tau_variant).
+// variant bit 2 (vgsim_set_tau_variant); bit 3 forces the warp kernel.
 cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant, int uniform_pp,
                        int *order_buf) {
     if ((long long)st.D.K * st.D.H + st.D.K >= (1 << 20)) return cudaErrorInvalidValue;  // owner id is packed in 20 bits
     const size_t stride = ((size_t)tau_layout(st.D, false, TAU_TEAM).bytes + 15) & ~(size_t)15;
-    int teams = (int)((227 * 1024 - TAU_CTA_TAIL) / stride), cap = 0;
+    int teams = (int)((227 * 1024 - TAU_CTA_TAIL) / stride);
     if (teams > 4) teams = 4;
     if (teams < 1) teams = 1;
-    bool team = (variant & 4) != 0, force_warp = (variant & 8) != 0;
-    // A/B knobs of the kernel mapping exist only in debug builds (-DVGSIM_DEBUG_KNOBS): the environment must not be able
-    // to change the mapping of a production run.  Measured dead ends they were used for are listed in DESIGN.md 4.1.
-#ifdef VGSIM_DEBUG_KNOBS
-#define VG_KNOB(name) getenv(name)
-#else
-#define VG_KNOB(name) ((const char *)nullptr)
-#endif
-    if (const char *e = VG_KNOB("VGSIM_TAU_KERNEL")) {
-        team = team || e[0] == 't';
-        force_warp = force_warp || e[0] == 'w';
-    }
+    bool team = (variant & 4) != 0;
+    const bool force_warp = (variant & 8) != 0;
     // Few replicates (all of them resident at once as 256-thread teams): the GPU is latency- not throughput-bound, and a
     // team walks a leap sooner than a single warp does -- 8.1x at the world shape (K = 100: the K x K x H force-of-
     // infection sums), 32 replicates x 1,200 leaps: 607 ms vs 4,948 ms (profiles/r1_k_*), same log bit for bit.
     const bool team_fits = stride + TAU_CTA_TAIL <= (size_t)227 * 1024;  // else only the warp kernel's leaner slice may fit
     if (!team && !force_warp && team_fits && st.R <= num_sms * teams) team = true;
     if (!team) {
-        int max_warps = 16;
-        if (const char *e = VG_KNOB("VGSIM_TAU_WARPS")) max_warps = atoi(e);
-        if (max_warps < 1) max_warps = 1;
-        WarpLayout L = warp_layout(st.D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024, max_warps);
+        WarpLayout L = warp_layout(st.D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024);
         L.gsync = (variant & 16) ? 0 : 3;  // lockstep generations: the warps of a CTA meet at leap start and before the draws
-        if (const char *e = VG_KNOB("VGSIM_TAU_SYNC")) L.gsync = atoi(e) & 7;
-        if (const char *e = VG_KNOB("VGSIM_TAU_SYNC_EVERY")) L.gevery = atoi(e) < 1 ? 1 : atoi(e);
-        if (const char *e = VG_KNOB("VGSIM_TAU_GROUP")) L.ggroup = atoi(e) < 0 ? 0 : atoi(e);
         const int LC = st.D.E + (st.D.K - 1) * st.D.S;     // local channels of a cell: 12-bit field of a queue entry
         if (L.nwarps >= 1 && st.D.K * st.D.H < 65536 && LC < 4000) {  // cell ids are held as uint16
             const WS ws = make_ws(L, st.D);
@@ -1341,13 +1314,10 @@ cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream
             int grid = (st.R + L.nwarps - 1) / L.nwarps;
             if (grid > num_sms) grid = num_sms;
             // size-sorted schedule (only useful with lockstep generations and more than one visit per CTA)
-            int sorted = L.gsync != 0 && order_buf != nullptr && st.R > grid * L.nwarps && !(variant & 32);
-            if (const char *e2 = VG_KNOB("VGSIM_TAU_SORT")) sorted = sorted && atoi(e2) != 0;
+            const bool sorted = L.gsync != 0 && order_buf != nullptr && st.R > grid * L.nwarps && !(variant & 32);
             if (sorted) {
-                int wmode = 0;  // debug A/B: 1 sorts by loop items (cells and present haplotypes) instead of cells
-                if (const char *e3 = VG_KNOB("VGSIM_TAU_WEIGHT")) wmode = atoi(e3);
-                tau_weight_kernel<<<(st.R * 32 + 255) / 256, 256, 0, stream>>>(st, order_buf, wmode);
-                tau_order_kernel<<<1, 1024, 0, stream>>>(st.R, (wmode == 1 ? 3 : 1) * st.D.K * st.D.H, order_buf, order_buf + st.R);
+                tau_weight_kernel<<<(st.R * 32 + 255) / 256, 256, 0, stream>>>(st, order_buf);
+                tau_order_kernel<<<1, 1024, 0, stream>>>(st.R, st.D.K * st.D.H, order_buf, order_buf + st.R);
             }
             const int *order = sorted ? order_buf + st.R : nullptr;
             void *args[] = {(void *)&st, (void *)&a, (void *)&L, (void *)&ws, (void *)&variant, (void *)&order};
@@ -1355,12 +1325,10 @@ cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream
         }
         // a single replicate's state does not fit one warp slice: fall through to the team kernel
     }
-    if (const char *e = VG_KNOB("VGSIM_TAU_CFG")) sscanf(e, "%dx%d", &teams, &cap);
-#undef VG_KNOB
-    if (teams >= 4) return launch_tau_cfg<4>(st, a, stream, num_sms, variant, cap);
-    if (teams == 3) return launch_tau_cfg<3>(st, a, stream, num_sms, variant, cap);
-    if (teams == 2) return launch_tau_cfg<2>(st, a, stream, num_sms, variant, cap);
-    return launch_tau_cfg<1>(st, a, stream, num_sms, variant, cap);
+    if (teams >= 4) return launch_tau_cfg<4>(st, a, stream, num_sms, variant);
+    if (teams == 3) return launch_tau_cfg<3>(st, a, stream, num_sms, variant);
+    if (teams == 2) return launch_tau_cfg<2>(st, a, stream, num_sms, variant);
+    return launch_tau_cfg<1>(st, a, stream, num_sms, variant);
 }
 
 cudaError_t tau_cta_end(unsigned long long *out1024, int reset) {

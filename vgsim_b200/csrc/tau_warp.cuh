@@ -16,22 +16,19 @@
 // The arithmetic is the team kernel's: same drift / propensity expressions (shared template functions),
 // same summation orders, same Philox addressing (owner, leap, retry|epoch, block), same samplers -- a leap
 // is a pure function of (state, seed), so the two kernels produce the same log.  The team kernel stays as a
-// parity tap (variant bit 2 / VGSIM_TAU_KERNEL=team).
+// parity tap (variant bit 2).
 #pragma once
-
-// compile-time A/B switches (defaults = the product; scripts/build_variant.sh builds the alternatives)
-#ifndef TW_B1B_ENUM
-#define TW_B1B_ENUM 1   // 0: dense pass over all K x H cells for the empty-cell drifts
-#endif
-#ifndef TW_PARK
-#define TW_PARK 1       // 0: split every drain round's totals at once
-#endif
-#ifndef TW_WIPE_CLEAR
-#define TW_WIPE_CLEAR 1 // the next row's wipe is also spread over the loop that clears the per-leap deltas (0: A/B)
-#endif
 
 namespace vg {
 
+// Slow-path queue entries per warp.  >= 64: half a round (two words per lane) must fit an empty queue.  Round 2, final
+// kernel (ms at t = 60 / 90 / 120): 96 entries 4.39 / 12.64 / 26.34, 112 entries 4.36 / 12.32 / 25.95 -- the out-migration
+// totals no longer read the per-leap Q table, so the queue gets the room
+constexpr int TW_QCAP = 112;
+// Warps (= replicates in flight) per CTA: 148 x 14 = 2072 replicates in flight.  ptxas gives a 448-thread CTA 128 registers
+// per thread (4 warps of an SM sub-partition share 16 K registers; 144 does not launch), so 15-16 warps would cost no
+// registers -- at T3 the shared-memory slice (14.4 KB + Q table) is the limit
+constexpr int TW_MAX_WARPS = 14;
 
 struct WarpLayout {
     int nwarps;        // warps (= replicates in flight) per CTA
@@ -55,7 +52,7 @@ struct WarpLayout {
 inline unsigned div_magic(int d) { return d > 1 ? (unsigned)((0x100000000ull + (unsigned)d - 1) / (unsigned)d) : 0u; }
 __device__ __forceinline__ int fdiv(int n, unsigned magic, int d) { return d > 1 ? (int)__umulhi((unsigned)n, magic) : n; }
 
-inline WarpLayout warp_layout(const Dims &D, bool par_shared, int pp0, int max_bytes, int max_warps) {
+inline WarpLayout warp_layout(const Dims &D, bool par_shared, int pp0, int max_bytes) {
     WarpLayout L;
     L.gsync = 0;
     L.gevery = 1;
@@ -65,12 +62,7 @@ inline WarpLayout warp_layout(const Dims &D, bool par_shared, int pp0, int max_b
     L.pp0 = pp0;
     L.use_masks = (H <= 64 && K <= 32) ? 1 : 0;
     L.has_eff = tau_eff_in_smem(D) ? 1 : 0;
-#ifndef VGSIM_TW_QCAP
-#define VGSIM_TW_QCAP 112   // >= 64: half a round (two words per lane) must fit an empty queue.  Round 2, final kernel
-                            // (ms at t = 60 / 90 / 120): 96 entries 4.39 / 12.64 / 26.34, 112 entries 4.36 / 12.32 / 25.95 -- the
-                            // out-migration totals no longer read the per-leap Q table, so the queue gets the room
-#endif
-    L.qcap = VGSIM_TW_QCAP;
+    L.qcap = TW_QCAP;
     L.xcap = 64;
     {
         const int NBT = (S + 3) >> 2, G2 = (S * (S - 1) + 3) >> 2, nbm = (3 * U + 3) >> 2, nbg = ((K - 1) * S + 3) >> 2;
@@ -127,13 +119,7 @@ inline WarpLayout warp_layout(const Dims &D, bool par_shared, int pp0, int max_b
     o = (o + 15) & ~15;
     L.o_warp0 = o;
     int nw = (max_bytes - o) / L.warp_bytes;
-    if (nw > max_warps) nw = max_warps;
-#ifndef VGSIM_TW_MAXWARPS
-#define VGSIM_TW_MAXWARPS 14
-#endif
-    if (nw > VGSIM_TW_MAXWARPS) nw = VGSIM_TW_MAXWARPS;  // 148 x 14 = 2072 replicates in flight.  ptxas gives a 448-thread CTA 128 registers per thread
-                           // (4 warps of an SM sub-partition share 16 K registers; 144 does not launch), so 15-16 warps
-                           // would cost no registers -- at T3 the shared-memory slice (14.4 KB + Q table) is the limit
+    if (nw > TW_MAX_WARPS) nw = TW_MAX_WARPS;
     L.nwarps = nw;
     if (nw >= 1) {  // what is left of the shared memory holds the per-leap table of Q[p, present h]
         int spare = ((max_bytes - o) / nw - L.warp_bytes) & ~15;
@@ -505,7 +491,7 @@ __device__ __forceinline__ double warp_min_d(double v) {
 // Drifts and tau (ChooseTau :2432-2450) of the warp's state; same sums as the team kernel's drifts_and_tau.
 template <class WSQ>
 __device__ __forceinline__ double w_drifts_and_tau(const Dims &D, const WSQ &s, const double *eff, int nhap, int nAct,
-                                                   RowWiper &wp, int wk, int n32, bool &dense_pass) {
+                                                   RowWiper &wp, int wk, int n32) {
     const int K = D.K, H = D.H, S = D.S, KS = K * S;
     const int lane = threadIdx.x & 31;
     // ---- A. pressure / return-flow sums per (deme, group): 8 lanes per sum, fixed butterfly
@@ -563,56 +549,52 @@ __device__ __forceinline__ double w_drifts_and_tau(const Dims &D, const WSQ &s, 
     //           is exact (their proposal is >= 1 and tau = min(1, ...)).  Pairs reached twice just repeat a candidate.
     // Sparse states (few infectious cells) enumerate; dense ones (measured: from ~1/8 of the cells on) are cheaper with
     // the plain pass over all K x H cells, which is skipped when qmax * (deme prevalence) < 1 in every deme.
-    if (TW_B1B_ENUM && nAct * 8 <= K * H) {
-    dense_pass = false;
-        {
-            const int U = D.U, n3 = 3 * U;
-            const int per = n3 > 0 ? 32 / n3 : 0;  // big cells handled per round
-            const double q3 = s.qmax[0] * (double)n3;
-            if (per > 0) {
+    if (nAct * 8 <= K * H) {
+        const int U = D.U, n3 = 3 * U;
+        const int per = n3 > 0 ? 32 / n3 : 0;  // big cells handled per round
+        const double q3 = s.qmax[0] * (double)n3;
+        if (per > 0) {
 #pragma unroll 1
-                for (int base = 0; base < nAct; base += 32) {
-                    const int a = base + lane;
-                    const int cell = a < nAct ? (int)s.act[a] : 0;
-                    const bool big = a < nAct && q3 * s.I[cell] >= 0.999;
-                    unsigned bm = __ballot_sync(0xffffffffu, big);
+            for (int base = 0; base < nAct; base += 32) {
+                const int a = base + lane;
+                const int cell = a < nAct ? (int)s.act[a] : 0;
+                const bool big = a < nAct && q3 * s.I[cell] >= 0.999;
+                unsigned bm = __ballot_sync(0xffffffffu, big);
 #pragma unroll 1
-                    while (bm) {
-                        // this round's big cells: the first `per` set bits
-                        const int slot = lane / n3, j = lane - slot * n3;
-                        unsigned m = bm;
-                        for (int k = 0; k < slot && m; k++) m &= m - 1;
-                        const int src_lane = m ? __ffs(m) - 1 : 0;
-                        const int bc = __shfl_sync(0xffffffffu, cell, src_lane);
-                        if (m && slot < per) {
-                            const int p = bc >> D.hshift, h = bc & (H - 1);
-                            const int u = j / 3, al = 1 + (j - u * 3);
-                            const int hn = h ^ (al << (2 * u));
-                            if (s.colcnt[hn] == 0) candidate(drift_I_cell(p * H + hn, D, s, eff), 0.0);
-                        }
-                        for (int k = 0; k < per && bm; k++) bm &= bm - 1;
-                    }
-                }
-            } else if (U > 0) {  // more than 10 sites: one big cell per round, its neighbours strided over the lanes
-#pragma unroll 1
-                for (int a = 0; a < nAct; a++) {
-                    const int bc = s.act[a];
-                    if (!(q3 * s.I[bc] >= 0.999)) continue;
-                    const int p = bc >> D.hshift, h = bc & (H - 1);
-                    for (int j = lane; j < n3; j += 32) {
+                while (bm) {
+                    // this round's big cells: the first `per` set bits
+                    const int slot = lane / n3, j = lane - slot * n3;
+                    unsigned m = bm;
+                    for (int k = 0; k < slot && m; k++) m &= m - 1;
+                    const int src_lane = m ? __ffs(m) - 1 : 0;
+                    const int bc = __shfl_sync(0xffffffffu, cell, src_lane);
+                    if (m && slot < per) {
+                        const int p = bc >> D.hshift, h = bc & (H - 1);
                         const int u = j / 3, al = 1 + (j - u * 3);
                         const int hn = h ^ (al << (2 * u));
                         if (s.colcnt[hn] == 0) candidate(drift_I_cell(p * H + hn, D, s, eff), 0.0);
                     }
+                    for (int k = 0; k < per && bm; k++) bm &= bm - 1;
+                }
+            }
+        } else if (U > 0) {  // more than 10 sites: one big cell per round, its neighbours strided over the lanes
+#pragma unroll 1
+            for (int a = 0; a < nAct; a++) {
+                const int bc = s.act[a];
+                if (!(q3 * s.I[bc] >= 0.999)) continue;
+                const int p = bc >> D.hshift, h = bc & (H - 1);
+                for (int j = lane; j < n3; j += 32) {
+                    const int u = j / 3, al = 1 + (j - u * 3);
+                    const int hn = h ^ (al << (2 * u));
+                    if (s.colcnt[hn] == 0) candidate(drift_I_cell(p * H + hn, D, s, eff), 0.0);
                 }
             }
         }
     } else {
-    int need = 0;
+        int need = 0;
 #pragma unroll 1
         for (int p = lane; p < K; p += 32) need |= s.qmax[0] * (double)s.tot[p] >= 0.999;
-        dense_pass = __any_sync(0xffffffffu, need) != 0;
-        if (dense_pass) {
+        if (__any_sync(0xffffffffu, need)) {
 #pragma unroll 1
             for (int i = lane; i < K * H; i += 32) {
                 wp.some(wk, n32);
@@ -761,14 +743,10 @@ __device__ __forceinline__ int tw_split_event(int owner, int kind, int e, const 
 }
 
 // One round (<= 32, taken from the end of the list) of parked aggregated totals: every lane splits one total, one event
-// per iteration.  TW_SPLIT_OUTLINE 1 keeps this walk out of the drain loop's instruction footprint (a call instead of
-// ~1,200 inlined SASS instructions): in dense states, where the drain is instruction-fetch bound, totals are rare.
-#ifndef TW_SPLIT_OUTLINE
-#define TW_SPLIT_OUTLINE 0
-#endif
+// per iteration.
 template <class WSQ>
-__device__ __forceinline__ void w_split_parked_impl(int *row, const Dims &D, const WSQ &s, const double *eff, const DrawGeom &g,
-                                                    const WarpLayout &L, PhiloxCtx &ctx, LeapTally &tr, DrawState &q) {
+__device__ __forceinline__ void w_split_parked(int *row, const Dims &D, const WSQ &s, const double *eff, const DrawGeom &g,
+                                               const WarpLayout &L, PhiloxCtx &ctx, LeapTally &tr, DrawState &q) {
     const int lane = threadIdx.x & 31;
     const int take = q.nsq < 32 ? q.nsq : 32;
     const int e = q.nsq - take + lane;
@@ -789,11 +767,6 @@ __device__ __forceinline__ void w_split_parked_impl(int *row, const Dims &D, con
     }
     q.nsq -= take;
     __syncwarp();
-}
-template <class WSQ>
-__device__ __noinline__ void w_split_parked(int *row, const Dims &D, const WSQ &s, const double *eff, const DrawGeom &g,
-                                            const WarpLayout &L, PhiloxCtx &ctx, LeapTally &tr, DrawState &q) {
-    w_split_parked_impl(row, D, s, eff, g, L, ctx, tr, q);
 }
 
 // Finish every queued draw and book the counts; all lanes walk the same code.
@@ -845,13 +818,7 @@ __device__ __forceinline__ void w_drain(int *row, const Dims &D, const WSQ &s, c
             __syncwarp();
         }
         // split one round of parked totals (taken from the end of the list)
-        if (q.nsq >= (TW_PARK ? 32 : 1) || (!more && final && q.nsq > 0)) {
-#if TW_SPLIT_OUTLINE
-            w_split_parked(row, D, s, eff, g, L, ctx, tr, q);
-#else
-            w_split_parked_impl(row, D, s, eff, g, L, ctx, tr, q);
-#endif
-        }
+        if (q.nsq >= 32 || (!more && final && q.nsq > 0)) w_split_parked(row, D, s, eff, g, L, ctx, tr, q);
         if (!more && !(final && q.nsq > 0)) break;
     }
     // ---- PTRS entries (lambda >= 10) sit at the top of the queue.  (A two-pass variant -- trial 0 with the quick
@@ -1050,21 +1017,13 @@ __device__ __forceinline__ void w_push(const RoundOut &ro, const WSQ &s, DrawSta
 // a CTA: weight = #infectious cells, sorted descending, consecutive groups of `nwarps` go to one CTA visit, and
 // the CTAs walk the groups boustrophedon (b, 2G-1-b, 2G+b, ...) so that every CTA gets the same mix of heavy and
 // light groups.  (KH below is the largest possible weight.)  Scheduling only: every replicate's result is a function of its own state and seed.
-__global__ void tau_weight_kernel(const DevState st, int *weight, int mode) {
-    const int lane = threadIdx.x & 31, K = st.D.K, H = st.D.H, KH = K * H;
+__global__ void tau_weight_kernel(const DevState st, int *weight) {
+    const int lane = threadIdx.x & 31, KH = st.D.K * st.D.H;
     const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (r >= st.R) return;
     int n = 0;
-    unsigned long long present = 0ull;  // haplotypes present anywhere (H <= 64)
-    for (int i = lane; i < KH; i += 32) {
-        const bool on = st.I[(size_t)r * KH + i] != 0;
-        n += on;
-        if (on) present |= 1ull << (i & (H - 1) & 63);
-    }
+    for (int i = lane; i < KH; i += 32) n += st.I[(size_t)r * KH + i] != 0;
     n = __reduce_add_sync(0xffffffffu, n);
-    unsigned lo = __reduce_or_sync(0xffffffffu, (unsigned)present), hi = __reduce_or_sync(0xffffffffu, (unsigned)(present >> 32));
-    // mode 1: items of the two long loops of a leap -- 2 draw blocks per cell + K drift sums per present haplotype
-    if (mode == 1 && H <= 64) n = 2 * n + K * (__popc(lo) + __popc(hi));
     if (lane == 0) weight[r] = n;
 }
 // one CTA: counting sort by weight (descending) into order[]
@@ -1088,11 +1047,7 @@ __global__ void __launch_bounds__(1024) tau_order_kernel(int R, int KH, const in
 }
 
 template <bool PROF, bool EFFS, bool MASKS>
-#ifdef VGSIM_TW_MAXNREG
-__global__ void __maxnreg__(VGSIM_TW_MAXNREG)
-#else
-__global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
-#endif
+__global__ void __launch_bounds__(TW_MAX_WARPS * 32, 1)
     tau_warp_kernel(const __grid_constant__ DevState st, const __grid_constant__ SimArgs a,
                     const __grid_constant__ WarpLayout L, const __grid_constant__ WSX<MASKS> s, const int variant,
                     const int *__restrict__ order) {
@@ -1103,7 +1058,6 @@ __global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
     const int n32 = D.Pp >> 3;  // 256-bit stores per log row
     // groups of 2 stores per lane per dense-loop round so that three dense loops (drift, feasibility, apply) cover a row
     const int wk = (((n32 + 31) / 32 + 3 * ((KH + 31) / 32) - 1) / (3 * ((KH + 31) / 32)) + 1) / 2;  // in groups of 2
-    const int wk2 = (((n32 + 31) / 32 + 2 * ((KH + 31) / 32) - 1) / (2 * ((KH + 31) / 32)) + 1) / 2;  // ... over two dense loops
     const bool prof = PROF;
     unsigned long long pc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     long long tmark = 0;
@@ -1240,9 +1194,7 @@ __global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
                         wp.idle();
                         pre_row = -1;
                     }
-                    bool dense_pass;
-                    double tau = w_drifts_and_tau(D, s, eff, nhap, nAct, wp, wk, n32, dense_pass);
-                    const int wkl = TW_WIPE_CLEAR ? 1 : (dense_pass ? wk : wk2);  // the empty-cell drift pass was skipped: its share of the wipe moves on
+                    double tau = w_drifts_and_tau(D, s, eff, nhap, nAct, wp, wk, n32);
                     TW_MARK(1)
                     if (meet && (gsync & 2)) TW_GEN_SYNC();
                     if (prof && lane == 0) tmark = clock64();
@@ -1256,7 +1208,7 @@ __global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
 #pragma unroll 1
                             for (int i = lane; i < n16; i += 32) {
                                 z[i] = make_int4(0, 0, 0, 0);
-                                if (TW_WIPE_CLEAR) wp.some(1, n32);
+                                wp.some(1, n32);
                             }
 #pragma unroll 1
                             for (int i = lane; i < KS; i += 32) s.dSx[i] = 0;
@@ -1322,7 +1274,7 @@ __global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
                         int bad = 0;
 #pragma unroll 1
                         for (int i = lane; i < KH; i += 32) {
-                            wp.some(wkl, n32);
+                            wp.some(1, n32);
                             const double sz = s.sizeD[i >> D.hshift];
                             const double Iv = s.I[i];
                             const double v = Iv + (double)s.chkI[i];
@@ -1370,7 +1322,7 @@ __global__ void __launch_bounds__(VGSIM_TW_MAXWARPS * 32, 1)
                     // ---- 5. apply (UpdateCompartmentCounts_tau, :2536-2593) fused with the list rebuild
 #pragma unroll 1
                     for (int i = lane; i < KS; i += 32) s.Sx[i] += (double)s.dSx[i];
-                    nAct = w_lists<WSX<MASKS>, true>(D, s, nhap, wp, wkl, n32);
+                    nAct = w_lists<WSX<MASKS>, true>(D, s, nhap, wp, 1, n32);
                     if (lane == 0) {
                         double *tau_tt = st.tau_tt + ((size_t)r * st.leap_cap + leaps) * 2;
                         tau_tt[0] = t;
