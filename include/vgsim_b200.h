@@ -5,7 +5,11 @@
  * below replaces one `BirthDeathModel` method or data member of the reference
  * (src/_BirthDeath.pyx, src/events.pxi, src/models.pxi), cited per function.  Plain pointers and
  * sizes only — no torch / numpy / CUDA types in any signature.  Every function returns 0 on
- * success, non-zero on failure; the message is available from vgsim_last_error().
+ * success, non-zero on failure; the message is available from vgsim_last_error().  The int64
+ * count functions (vgsim_num_lockdowns, vgsim_tree_size, vgsim_num_mutations,
+ * vgsim_num_migrations) return -1 on failure, e.g. for a replicate index outside [0, R), and 0
+ * when there is nothing to count (no genealogy yet).  Every entry point that takes a replicate
+ * index fails with "replicate out of range" outside [0, R).
  *
  * A handle owns R independent replicates of one model shape (sites U -> H = 4^U haplotypes,
  * K demes, S susceptibility groups) on one CUDA device: compartment state, per-replicate event

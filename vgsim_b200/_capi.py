@@ -108,6 +108,13 @@ def _ck(rc):
         raise VgsimError(lib.vgsim_last_error().decode())
 
 
+def _count(n):
+    """Result of an int64 count function: -1 is an error (e.g. a replicate out of range)."""
+    if n < 0:
+        raise VgsimError(lib.vgsim_last_error().decode())
+    return int(n)
+
+
 def _p(a):
     return None if a is None else a.ctypes.data_as(c_void_p)
 
@@ -339,20 +346,20 @@ class Handle:
         _ck(lib.vgsim_set_event_log(self._h, replicate, _p(chain), chain.shape[1], _p(I_end)))
 
     def get_lockdowns(self, replicate=0):
-        n = int(lib.vgsim_num_lockdowns(self._h, replicate))
+        n = _count(lib.vgsim_num_lockdowns(self._h, replicate))
         st, pop, t = np.zeros(n, np.int64), np.zeros(n, np.int64), np.zeros(n, np.float64)
         _ck(lib.vgsim_get_lockdowns(self._h, replicate, _p(st), _p(pop), _p(t)))
         return st, pop, t
 
     def get_tree(self, replicate=0):
-        n = int(lib.vgsim_tree_size(self._h, replicate))
+        n = _count(lib.vgsim_tree_size(self._h, replicate))
         parent, pop, t = np.zeros(n, np.int64), np.zeros(n, np.int64), np.zeros(n, np.float64)
         if n:
             _ck(lib.vgsim_get_tree(self._h, replicate, _p(parent), _p(pop), _p(t)))
         return parent, pop, t
 
     def get_mutations(self, replicate=0):
-        n = int(lib.vgsim_num_mutations(self._h, replicate))
+        n = _count(lib.vgsim_num_mutations(self._h, replicate))
         node, AS, DS, site = (np.zeros(n, np.int64) for _ in range(4))
         t = np.zeros(n, np.float64)
         if n:
@@ -360,7 +367,7 @@ class Handle:
         return node, AS, DS, site, t
 
     def get_migrations(self, replicate=0):
-        n = int(lib.vgsim_num_migrations(self._h, replicate))
+        n = _count(lib.vgsim_num_migrations(self._h, replicate))
         node, oldp, newp = (np.zeros(n, np.int64) for _ in range(3))
         t = np.zeros(n, np.float64)
         if n:
@@ -420,8 +427,7 @@ class Handle:
 def test_poisson(lam, seed=1):
     lam = np.ascontiguousarray(lam, np.float64)
     out = np.zeros(lam.shape, np.int64)
-    if lib.vgsim_test_poisson(_p(lam), lam.size, seed, _p(out)) != 0:
-        raise VgsimError("vgsim_test_poisson failed")
+    _ck(lib.vgsim_test_poisson(_p(lam), lam.size, seed, _p(out)))
     return out
 
 
@@ -430,8 +436,7 @@ def test_hypergeometric(good, bad, sample, raw_words):
     raw = np.ascontiguousarray(raw_words, np.uint64)
     out = np.zeros(good.shape, np.int64)
     used = np.zeros(1, np.int64)
-    if lib.vgsim_test_hypergeometric(_p(good), _p(bad), _p(sample), good.size, _p(raw), raw.size, _p(out), _p(used)) != 0:
-        raise VgsimError("vgsim_test_hypergeometric failed")
+    _ck(lib.vgsim_test_hypergeometric(_p(good), _p(bad), _p(sample), good.size, _p(raw), raw.size, _p(out), _p(used)))
     return out, int(used[0])
 
 
@@ -441,7 +446,6 @@ def test_choose(w, x, skip=-1, small=False):
     x = np.ascontiguousarray(x, np.float64)
     idx = np.zeros(x.shape, np.int64)
     before, wsel, resid = (np.zeros(x.shape, np.float64) for _ in range(3))
-    if lib.vgsim_test_choose(_p(w), w.size, _p(x), x.size, int(skip), 1 if small else 0, _p(idx), _p(before), _p(wsel),
-                             _p(resid)) != 0:
-        raise VgsimError("vgsim_test_choose failed")
+    _ck(lib.vgsim_test_choose(_p(w), w.size, _p(x), x.size, int(skip), 1 if small else 0, _p(idx), _p(before), _p(wsel),
+                              _p(resid)))
     return idx, before, wsel, resid

@@ -4,54 +4,19 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 #include "../../include/vgsim_b200.h"
 #include "common.cuh"
-#include "handle.h"
+#include "host.h"
 
 using namespace vg;
 
 static thread_local std::string g_err;
-static int fail(const std::string &m) {
+int vg::fail(const std::string &m) {
     g_err = m;
     return 1;
-}
-#define HOST_SYNC(h)                                                    \
-    do {                                                                \
-        if (!(h)->async_host) CK(cudaStreamSynchronize((h)->stream));   \
-    } while (0)
-#define CK(call)                                                                                   \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess)                                                                     \
-            return fail(std::string(#call) + ": " + cudaGetErrorString(e_));                       \
-    } while (0)
-
-struct vgsim_handle_s : public Handle {};
-
-int vgsim_set_error(const char *msg) {
-    g_err = msg;
-    return 1;
-}
-
-template <class T>
-static int dalloc(Handle *h, T **p, size_t n) {
-    void *q = nullptr;
-    if (n == 0) n = 1;
-    cudaError_t e = cudaMalloc(&q, n * sizeof(T));
-    if (e != cudaSuccess) return fail(std::string("cudaMalloc: ") + cudaGetErrorString(e));
-    e = cudaMemsetAsync(q, 0, n * sizeof(T), h->stream);
-    if (e != cudaSuccess) return fail(std::string("cudaMemset: ") + cudaGetErrorString(e));
-    h->allocs.push_back(q);
-    *p = (T *)q;
-    return 0;
-}
-static void dfree(Handle *h, void *p) {
-    if (!p) return;
-    auto it = std::find(h->allocs.begin(), h->allocs.end(), p);
-    if (it != h->allocs.end()) h->allocs.erase(it);
-    cudaFree(p);
 }
 
 extern "C" {
@@ -71,17 +36,16 @@ int vgsim_create(int sites, int K, int S, int n_replicates, int n_param_points, 
                     cudaGetErrorString(e));
     if (device < 0) CK(cudaGetDevice(&device));
     CK(cudaSetDevice(device));
-    vgsim_handle_s *h = new vgsim_handle_s();
+    std::unique_ptr<vgsim_handle_s, int (*)(vgsim_handle)> owner(new vgsim_handle_s(), vgsim_destroy);  // on failure
+    vgsim_handle_s *h = owner.get();
     h->device = device;
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     h->num_sms = prop.multiProcessorCount;
     h->D = make_dims(sites, K, S);
     const Dims &D = h->D;
-    if ((long long)K * (K - 1) * S * D.H + (long long)K * D.PD > 2000000000LL) {
-        delete h;
+    if ((long long)K * (K - 1) * S * D.H + (long long)K * D.PD > 2000000000LL)
         return fail("too many reaction channels for 32-bit channel indices");
-    }
     h->R = n_replicates;
     h->n_pp = n_param_points;
     h->hp.resize(n_param_points);
@@ -105,19 +69,15 @@ int vgsim_create(int sites, int K, int S, int n_replicates, int n_param_points, 
         dalloc(h, &st.eff, R * K * K) || dalloc(h, &st.ceff, R * K) || dalloc(h, &st.maxEBM, R * K) ||
         dalloc(h, &st.time, R) || dalloc(h, &st.counters, R * NCOUNT) || dalloc(h, &st.epoch, R) ||
         dalloc(h, &st.err, R) || dalloc(h, &st.loc_n, R) || dalloc(h, &st.ev_base, R) || dalloc(h, &st.dense_base, R) ||
-        dalloc(h, &st.sp_n, R) || dalloc(h, &st.rate_tot, 2 * R)) {
-        vgsim_destroy(h);
+        dalloc(h, &st.sp_n, R) || dalloc(h, &st.rate_tot, 2 * R))
         return 1;
-    }
     st.params = params;
     st.rep_pp = rep_pp;
     st.seeds = seeds;
     st.loc_cap = 64 + 16 * K;  // a deme flips its lockdown on and off a few times per wave; overflow sets a sticky error bit
     if (dalloc(h, &st.loc_sp, R * st.loc_cap) || dalloc(h, &st.loc_t, R * st.loc_cap) ||
-        dalloc(h, &h->summaries, R * VGSIM_NSUMMARY) || dalloc(h, &h->tau_order, 2 * R) || dalloc(h, &h->work, 4)) {
-        vgsim_destroy(h);
+        dalloc(h, &h->summaries, R * VGSIM_NSUMMARY) || dalloc(h, &h->tau_order, 2 * R) || dalloc(h, &h->work, 4))
         return 1;
-    }
     // default state: everyone susceptible in group 0, sizes 1e6 (reference :201-204)
     std::vector<long long> Sx(R * K * S, 0);
     for (size_t i = 0; i < R * K; i++) Sx[i * S] = 1000000;
@@ -126,7 +86,7 @@ int vgsim_create(int sites, int K, int S, int n_replicates, int n_param_points, 
     for (size_t i = 0; i < R; i++) sd[i] = i;
     CK(cudaMemcpyAsync(seeds, sd.data(), R * 8, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    *out = h;
+    *out = owner.release();
     return 0;
 }
 
@@ -304,10 +264,9 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
         for (int p = 0; p < K; p++) mask[p] = cd_reset_mask[p] != 0;
     else if (P.uploaded && !contact_density)
         std::fill(mask.begin(), mask.end(), 0);
-    int *dmask;
-    double *dcd;
-    CK(cudaMalloc(&dmask, K * 4));
-    CK(cudaMalloc(&dcd, K * 8));
+    Scratch<int> dmask;
+    Scratch<double> dcd;
+    if (dmask.alloc(K) || dcd.alloc(K)) return 1;
     CK(cudaMemcpyAsync(dmask, mask.data(), K * 4, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(dcd, P.cd.data(), K * 8, cudaMemcpyHostToDevice, h->stream));
     int n = h->R * K;
@@ -315,8 +274,6 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
     h->launches++;
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
-    cudaFree(dmask);
-    cudaFree(dcd);
     P.uploaded = true;
     return 0;
 }
@@ -439,13 +396,11 @@ template <class T>
 static int grow2d(Handle *h, T **buf, long long old_cap, long long new_cap, long long keep, size_t w) {
     T *nb;
     if (dalloc(h, &nb, (size_t)h->R * new_cap * w)) return 1;
-    if (*buf && keep > 0) {
-        cudaError_t e = cudaMemcpy2DAsync(nb, new_cap * w * sizeof(T), *buf, old_cap * w * sizeof(T),
-                                          keep * w * sizeof(T), h->R, cudaMemcpyDeviceToDevice, h->stream);
-        if (e != cudaSuccess) return fail(std::string("cudaMemcpy2D: ") + cudaGetErrorString(e));
-    }
+    if (*buf && keep > 0)
+        CK(cudaMemcpy2DAsync(nb, new_cap * w * sizeof(T), *buf, old_cap * w * sizeof(T), keep * w * sizeof(T), h->R,
+                             cudaMemcpyDeviceToDevice, h->stream));
     if (*buf) {
-        cudaStreamSynchronize(h->stream);
+        CK(cudaStreamSynchronize(h->stream));
         dfree(h, *buf);
     }
     *buf = nb;
@@ -471,11 +426,10 @@ static int ensure_leap_cap(Handle *h, long long need) {  // tau_tt and the archi
         int *nb;
         if (dalloc(h, &nb, (size_t)h->R * (nc + 1))) return 1;
         if (st.sp_off && h->leap_bound > 0)
-            if (cudaMemcpy2DAsync(nb, (nc + 1) * 4, st.sp_off, (st.leap_cap + 1) * 4, (h->leap_bound + 1) * 4, h->R,
-                                  cudaMemcpyDeviceToDevice, h->stream) != cudaSuccess)
-                return fail("cudaMemcpy2D (archive offsets)");
+            CK(cudaMemcpy2DAsync(nb, (nc + 1) * 4, st.sp_off, (st.leap_cap + 1) * 4, (h->leap_bound + 1) * 4, h->R,
+                                 cudaMemcpyDeviceToDevice, h->stream));
         if (st.sp_off) {
-            cudaStreamSynchronize(h->stream);
+            CK(cudaStreamSynchronize(h->stream));
             dfree(h, st.sp_off);
         }
         st.sp_off = nb;
@@ -735,25 +689,21 @@ int64_t vgsim_prop_num(vgsim_handle h) { return h->D.P; }
 
 int vgsim_propensities(vgsim_handle h, int replicate, double *out, double *dI, double *dS, double *tau) {
     CK(cudaSetDevice(h->device));
-    if (replicate < 0 || replicate >= h->R) return fail("replicate out of range");
+    if (check_replicate(h, replicate)) return 1;
     if (!h->hp[0].uploaded) return fail("parameters were not uploaded");
     const Dims &D = h->D;
     // like PrintPropensities: UpdateAllRates on the CURRENT state (no FirstInfection, no lockdown check)
     cudaError_t e = launch_refresh(h->st, h->stream);
     if (e != cudaSuccess) return fail(std::string("refresh kernel: ") + cudaGetErrorString(e));
-    double *buf;
+    Scratch<double> buf;
     size_t n = (size_t)D.P + (size_t)D.K * D.H + (size_t)D.K * D.S + 1;
-    CK(cudaMalloc(&buf, n * 8));
+    if (buf.alloc(n)) return 1;
     e = launch_propensities(h->st, replicate, buf, buf + D.P, buf + D.P + D.K * D.H, buf + n - 1, h->stream);
     h->launches += 2;
-    if (e != cudaSuccess) {
-        cudaFree(buf);
-        return fail(std::string("propensity kernel: ") + cudaGetErrorString(e));
-    }
+    if (e != cudaSuccess) return fail(std::string("propensity kernel: ") + cudaGetErrorString(e));
     std::vector<double> hb(n);
     CK(cudaMemcpyAsync(hb.data(), buf, n * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    cudaFree(buf);
     if (out) memcpy(out, hb.data(), (size_t)D.P * 8);
     if (dI) memcpy(dI, hb.data() + D.P, (size_t)D.K * D.H * 8);
     if (dS) memcpy(dS, hb.data() + D.P + D.K * D.H, (size_t)D.K * D.S * 8);
@@ -764,22 +714,19 @@ int vgsim_propensities(vgsim_handle h, int replicate, double *out, double *dI, d
 int vgsim_rates(vgsim_handle h, int replicate, double *A, double *eff, double *maxEBM, double *ev, double *hapPopRate,
                 double *popRate, double *migPopRate, double *totals) {
     CK(cudaSetDevice(h->device));
-    if (replicate < 0 || replicate >= h->R) return fail("replicate out of range");
+    if (check_replicate(h, replicate)) return 1;
     if (!h->hp[0].uploaded) return fail("parameters were not uploaded");
     const Dims &D = h->D;
     const int K = D.K, H = D.H;
     cudaError_t e = launch_refresh(h->st, h->stream);
     if (e != cudaSuccess) return fail(std::string("refresh kernel: ") + cudaGetErrorString(e));
     size_t n = (size_t)K * H * 4 + (size_t)K * H + K + K + 2;
-    double *buf;
-    CK(cudaMalloc(&buf, n * 8));
+    Scratch<double> buf;
+    if (buf.alloc(n)) return 1;
     e = launch_rates_tap(h->st, replicate, buf, buf + K * H * 4, buf + K * H * 5, buf + K * H * 5 + K,
                          buf + K * H * 5 + 2 * K, h->stream);
     h->launches += 2;
-    if (e != cudaSuccess) {
-        cudaFree(buf);
-        return fail(std::string("rates kernel: ") + cudaGetErrorString(e));
-    }
+    if (e != cudaSuccess) return fail(std::string("rates kernel: ") + cudaGetErrorString(e));
     std::vector<double> hb(n);
     CK(cudaMemcpyAsync(hb.data(), buf, n * 8, cudaMemcpyDeviceToHost, h->stream));
     int pp;
@@ -788,7 +735,6 @@ int vgsim_rates(vgsim_handle h, int replicate, double *A, double *eff, double *m
     if (maxEBM) CK(cudaMemcpyAsync(maxEBM, h->st.maxEBM + (size_t)replicate * K, (size_t)K * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (A) CK(cudaMemcpy(A, h->st.params + (size_t)pp * D.blob + D.o_A, (size_t)K * 8, cudaMemcpyDeviceToHost));
-    cudaFree(buf);
     if (ev) memcpy(ev, hb.data(), (size_t)K * H * 4 * 8);
     if (hapPopRate) memcpy(hapPopRate, hb.data() + K * H * 4, (size_t)K * H * 8);
     if (popRate) memcpy(popRate, hb.data() + K * H * 5, (size_t)K * 8);
@@ -814,7 +760,7 @@ static int fetch_counters(Handle *h, int r, long long *c) {
 
 int vgsim_get_event_log(vgsim_handle h, int r, double *out, int64_t n) {
     CK(cudaSetDevice(h->device));
-    if (r < 0 || r >= h->R) return fail("replicate out of range");
+    if (check_replicate(h, r)) return 1;
     long long c[NCOUNT];
     if (fetch_counters(h, r, c)) return 1;
     if (n != c[C_EVPTR]) return fail("event count mismatch (expected counters[9])");
@@ -848,7 +794,7 @@ int vgsim_get_event_log(vgsim_handle h, int r, double *out, int64_t n) {
 
 int vgsim_get_tau_log(vgsim_handle h, int r, int64_t leaps, int32_t *counts, double *time_tau) {
     CK(cudaSetDevice(h->device));
-    if (r < 0 || r >= h->R) return fail("replicate out of range");
+    if (check_replicate(h, r)) return 1;
     long long c[NCOUNT];
     if (fetch_counters(h, r, c)) return 1;
     if (leaps != c[C_LEAPS]) return fail("leap count mismatch (expected counters[10])");
@@ -929,16 +875,20 @@ int vgsim_get_multievents(vgsim_handle h, int r, int64_t n, int64_t *num, double
     return 0;
 }
 
+static int lockdown_count(Handle *h, int r, int *n) {
+    if (check_replicate(h, r)) return 1;
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(n, h->st.loc_n + r, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
 int64_t vgsim_num_lockdowns(vgsim_handle h, int r) {
-    cudaSetDevice(h->device);
     int n = 0;
-    cudaMemcpyAsync(&n, h->st.loc_n + r, 4, cudaMemcpyDeviceToHost, h->stream);
-    cudaStreamSynchronize(h->stream);
-    return n;
+    return lockdown_count(h, r, &n) ? -1 : n;
 }
 int vgsim_get_lockdowns(vgsim_handle h, int r, int64_t *state, int64_t *pop, double *time) {
-    CK(cudaSetDevice(h->device));
-    int n = (int)vgsim_num_lockdowns(h, r);
+    int n = 0;
+    if (lockdown_count(h, r, &n)) return 1;
     if (n == 0) return 0;
     std::vector<int> sp(n);
     CK(cudaMemcpyAsync(sp.data(), h->st.loc_sp + (size_t)r * h->st.loc_cap, n * 4, cudaMemcpyDeviceToHost, h->stream));
@@ -959,40 +909,28 @@ int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step
     if (step_num < 1) return fail("epidemic curves: step_num must be >= 1");
     const Dims &D = h->D;
     const size_t np = (size_t)rep_count * (step_num + 1), KH = (size_t)D.K * D.H, KS = (size_t)D.K * D.S;
-    long long *d_inf = nullptr, *d_sus = nullptr, *d_rem = nullptr, *d_smp = nullptr;
-    double *d_tp = nullptr;
-    int *d_lp = nullptr;
-    int rc = 0;
-    if (infectious && !rc) rc = dalloc(h, &d_inf, np * KH);
-    if (susceptible && !rc) rc = dalloc(h, &d_sus, np * KS);
-    if (removed && !rc) rc = dalloc(h, &d_rem, np * KH);
-    if (sampled && !rc) rc = dalloc(h, &d_smp, np * KH);
-    if (time_points && !rc) rc = dalloc(h, &d_tp, np);
-    if (last_point && !rc) rc = dalloc(h, &d_lp, (size_t)rep_count);
-    cudaError_t e = cudaSuccess;
-    if (!rc) {
-        next_timer(h);
-        cudaEventRecord(h->ev_k0, h->stream);  // vgsim_last_kernel_ms then reports this kernel
-        e = launch_curves(h->st, rep_first, rep_count, step_num, d_inf, d_sus, d_rem, d_smp, d_tp, d_lp, h->stream, h->num_sms);
-        cudaEventRecord(h->ev_k1, h->stream);
-        h->ev_valid = true;
-        h->launches++;
-    }
-    auto back = [&](void *dst, const void *src, size_t bytes) {
-        if (dst && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->stream);
-    };
-    if (!rc) {
-        back(infectious, d_inf, np * KH * 8);
-        back(susceptible, d_sus, np * KS * 8);
-        back(removed, d_rem, np * KH * 8);
-        back(sampled, d_smp, np * KH * 8);
-        back(time_points, d_tp, np * 8);
-        back(last_point, d_lp, (size_t)rep_count * 4);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    }
-    dfree(h, d_inf); dfree(h, d_sus); dfree(h, d_rem); dfree(h, d_smp); dfree(h, d_tp); dfree(h, d_lp);
-    if (rc) return rc;
+    // every output the kernel is given is written in full: the buffers need no zero fill
+    Scratch<long long> d_inf, d_sus, d_rem, d_smp;
+    Scratch<double> d_tp;
+    Scratch<int> d_lp;
+    if ((infectious && d_inf.alloc(np * KH)) || (susceptible && d_sus.alloc(np * KS)) || (removed && d_rem.alloc(np * KH)) ||
+        (sampled && d_smp.alloc(np * KH)) || (time_points && d_tp.alloc(np)) || (last_point && d_lp.alloc(rep_count)))
+        return 1;
+    next_timer(h);
+    CK(cudaEventRecord(h->ev_k0, h->stream));  // vgsim_last_kernel_ms then reports this kernel
+    cudaError_t e = launch_curves(h->st, rep_first, rep_count, step_num, d_inf, d_sus, d_rem, d_smp, d_tp, d_lp, h->stream,
+                                  h->num_sms);
+    CK(cudaEventRecord(h->ev_k1, h->stream));
+    h->ev_valid = true;
+    h->launches++;
     if (e != cudaSuccess) return fail(std::string("epidemic curves: ") + cudaGetErrorString(e));
+    if (infectious) CK(cudaMemcpyAsync(infectious, d_inf, np * KH * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (susceptible) CK(cudaMemcpyAsync(susceptible, d_sus, np * KS * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (removed) CK(cudaMemcpyAsync(removed, d_rem, np * KH * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (sampled) CK(cudaMemcpyAsync(sampled, d_smp, np * KH * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (time_points) CK(cudaMemcpyAsync(time_points, d_tp, np * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (last_point) CK(cudaMemcpyAsync(last_point, d_lp, (size_t)rep_count * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
@@ -1178,7 +1116,7 @@ int vgsim_summaries(vgsim_handle h, double *out) {
 
 int vgsim_set_event_log(vgsim_handle h, int r, const double *in, int64_t n, const int64_t *I_end) {
     CK(cudaSetDevice(h->device));
-    if (r < 0 || r >= h->R) return fail("replicate out of range");
+    if (check_replicate(h, r)) return 1;
     const Dims &D = h->D;
     if (ensure_ev_cap(h, n > h->ev_bound ? n : h->ev_bound)) return 1;
     std::vector<double> t(n);

@@ -25,7 +25,7 @@
 #include "../../include/vgsim_b200.h"
 #include "common.cuh"
 #include "logrec.cuh"
-#include "handle.h"
+#include "host.h"
 #include "genrng.cuh"
 
 namespace vg {
@@ -533,64 +533,23 @@ __global__ void __launch_bounds__(128) genealogy_kernel(DevState st, GenArgs ga)
 
 using namespace vg;
 
-static thread_local std::string g_gerr;
-extern "C" const char *vgsim_last_error(void);
-
-struct vgsim_handle_s : public Handle {};
-
 namespace {
 
-template <class T>
-int galloc(Handle *h, T **p, size_t n) {
-    void *q = nullptr;
-    if (n == 0) n = 1;
-    if (cudaMalloc(&q, n * sizeof(T)) != cudaSuccess) return 1;
-    h->allocs.push_back(q);
-    *p = (T *)q;
-    return 0;
-}
-void gfree(Handle *h, void *p) {
-    if (!p) return;
-    auto it = std::find(h->allocs.begin(), h->allocs.end(), p);
-    if (it != h->allocs.end()) h->allocs.erase(it);
-    cudaFree(p);
-}
 void free_gen(Handle *h) {
     GenealogyBuffers &G = h->gen;
     void *ptrs[] = {G.node_off, G.parent, G.pop, G.time, G.mut_off, G.mig_off, G.mut_n, G.mig_n, G.mut_node, G.mut_hap,
                     G.mut_nhap, G.mut_time, G.mig_node, G.mig_old, G.mig_new, G.mig_time, G.arena_off, G.arena,
                     G.cell_hdr, G.n_nodes, G.scratch};
-    for (void *p : ptrs) gfree(h, p);
+    for (void *p : ptrs) dfree(h, p);
     G = GenealogyBuffers();
 }
 
-}  // namespace
-
-extern int vgsim_set_error(const char *msg);
-
-extern "C" {
-
-int vgsim_genealogy(vgsim_handle h, const uint64_t *seeds, const double *uniform_stream, const int64_t *stream_offsets,
-                    int raw_words) {
-    if (cudaSetDevice(h->device) != cudaSuccess) return vgsim_set_error("cudaSetDevice failed");
-    if (!h->st.first_simulation) return vgsim_set_error("nothing was simulated");
+// One replay of every replicate's log into new output buffers whose side tables are `table_scale` times the default
+// size; `ga` brings the caller's seeds or uniform stream.  *overflow: the side tables of some replicate overflowed (its
+// error bit is cleared again).
+int replay(Handle *h, const std::vector<long long> &ctr, long long table_scale, GenArgs ga, bool *overflow) {
     const Dims &D = h->D;
     const int R = h->R;
-    std::vector<long long> ctr((size_t)R * NCOUNT);
-    cudaStreamSynchronize(h->stream);
-    if (cudaMemcpy(ctr.data(), h->st.counters, ctr.size() * 8, cudaMemcpyDeviceToHost) != cudaSuccess)
-        return vgsim_set_error("counter read-back failed");
-    // The mutation / migration side tables grow with rate x branch length, not with the sample count (the reference
-    // appends to std::vectors, src/models.pxi): start from a size that covers the usual case and, if a replicate
-    // overflows, run the replay again with 8x larger tables.  The replay rewinds the infectious counts in place (quirk
-    // Q9), so they are saved first and put back before a retry.
-    long long *I_saved = nullptr;
-    const size_t I_n = (size_t)R * D.K * D.H;
-    if (cudaMalloc(&I_saved, I_n * 8) != cudaSuccess) return vgsim_set_error("cudaMalloc failed");
-    cudaMemcpyAsync(I_saved, h->st.I, I_n * 8, cudaMemcpyDeviceToDevice, h->stream);
-    long long table_scale = 1;
-    for (int attempt = 0;; attempt++, table_scale *= 8) {
-    if (attempt > 0) cudaMemcpyAsync(h->st.I, I_saved, I_n * 8, cudaMemcpyDeviceToDevice, h->stream);
     free_gen(h);
     GenealogyBuffers &G = h->gen;
     G.h_node_off.assign(R + 1, 0);
@@ -605,27 +564,22 @@ int vgsim_genealogy(vgsim_handle h, const uint64_t *seeds, const double *uniform
         G.h_mut_off[r + 1] = G.h_mut_off[r] + (sC >= 2 ? (8 * sC + 64) * table_scale : 0);
         G.h_mig_off[r + 1] = G.h_mig_off[r] + (sC >= 2 ? (3 * sC + 8) * table_scale : 0);
         arena_off[r + 1] = arena_off[r] + (sC >= 2 ? 2 * (2 * sC + 4 * KH) : 0);
-        if (2 * sC + 4 * KH > 1000000000LL) return vgsim_set_error("sample count too large for int32 lineage arena");
+        if (2 * sC + 4 * KH > 1000000000LL) return fail("sample count too large for int32 lineage arena");
     }
     G.total_nodes = G.h_node_off[R];
-    unsigned long long *dseeds = nullptr;
-    double *dstream = nullptr;
-    long long *doff = nullptr, *dused = nullptr;
-    if (galloc(h, &G.node_off, R + 1) || galloc(h, &G.mut_off, R + 1) || galloc(h, &G.mig_off, R + 1) ||
-        galloc(h, &G.arena_off, R + 1) || galloc(h, &G.parent, G.total_nodes) || galloc(h, &G.pop, G.total_nodes) ||
-        galloc(h, &G.time, G.total_nodes) || galloc(h, &G.scratch, G.total_nodes) || galloc(h, &G.arena, arena_off[R]) ||
-        galloc(h, &G.cell_hdr, (size_t)R * KH * 3) || galloc(h, &G.n_nodes, R) || galloc(h, &G.mut_n, R) ||
-        galloc(h, &G.mig_n, R) || galloc(h, &G.mut_node, G.h_mut_off[R]) || galloc(h, &G.mut_hap, G.h_mut_off[R]) ||
-        galloc(h, &G.mut_nhap, G.h_mut_off[R]) || galloc(h, &G.mut_time, G.h_mut_off[R]) ||
-        galloc(h, &G.mig_node, G.h_mig_off[R]) || galloc(h, &G.mig_old, G.h_mig_off[R]) ||
-        galloc(h, &G.mig_new, G.h_mig_off[R]) || galloc(h, &G.mig_time, G.h_mig_off[R]))
-        return vgsim_set_error("cudaMalloc failed for the genealogy buffers");
-    cudaMemcpyAsync(G.node_off, G.h_node_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream);
-    cudaMemcpyAsync(G.mut_off, G.h_mut_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream);
-    cudaMemcpyAsync(G.mig_off, G.h_mig_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream);
-    cudaMemcpyAsync(G.arena_off, arena_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream);
-    GenArgs ga;
-    memset(&ga, 0, sizeof(ga));
+    if (dalloc(h, &G.node_off, R + 1) || dalloc(h, &G.mut_off, R + 1) || dalloc(h, &G.mig_off, R + 1) ||
+        dalloc(h, &G.arena_off, R + 1) || dalloc(h, &G.parent, G.total_nodes) || dalloc(h, &G.pop, G.total_nodes) ||
+        dalloc(h, &G.time, G.total_nodes) || dalloc(h, &G.scratch, G.total_nodes) || dalloc(h, &G.arena, arena_off[R]) ||
+        dalloc(h, &G.cell_hdr, (size_t)R * KH * 3) || dalloc(h, &G.n_nodes, R) || dalloc(h, &G.mut_n, R) ||
+        dalloc(h, &G.mig_n, R) || dalloc(h, &G.mut_node, G.h_mut_off[R]) || dalloc(h, &G.mut_hap, G.h_mut_off[R]) ||
+        dalloc(h, &G.mut_nhap, G.h_mut_off[R]) || dalloc(h, &G.mut_time, G.h_mut_off[R]) ||
+        dalloc(h, &G.mig_node, G.h_mig_off[R]) || dalloc(h, &G.mig_old, G.h_mig_off[R]) ||
+        dalloc(h, &G.mig_new, G.h_mig_off[R]) || dalloc(h, &G.mig_time, G.h_mig_off[R]))
+        return 1;
+    CK(cudaMemcpyAsync(G.node_off, G.h_node_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(G.mut_off, G.h_mut_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(G.mig_off, G.h_mig_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(G.arena_off, arena_off.data(), (R + 1) * 8, cudaMemcpyHostToDevice, h->stream));
     ga.node_off = G.node_off;
     ga.parent = G.parent;
     ga.pop = G.pop;
@@ -647,86 +601,106 @@ int vgsim_genealogy(vgsim_handle h, const uint64_t *seeds, const double *uniform
     ga.n_nodes = G.n_nodes;
     ga.mut_n = G.mut_n;
     ga.mig_n = G.mig_n;
-    ga.raw_words = raw_words;
-    if (seeds) {
-        if (galloc(h, &dseeds, R)) return vgsim_set_error("cudaMalloc failed");
-        cudaMemcpyAsync(dseeds, seeds, (size_t)R * 8, cudaMemcpyHostToDevice, h->stream);
-        ga.new_seeds = dseeds;
-    }
-    if (uniform_stream) {
-        if (!stream_offsets) return vgsim_set_error("stream_offsets is required with uniform_stream");
-        long long n = stream_offsets[R];
-        if (galloc(h, &dstream, n) || galloc(h, &doff, R + 1) || galloc(h, &dused, R))
-            return vgsim_set_error("cudaMalloc failed");
-        cudaMemcpyAsync(dstream, uniform_stream, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream);
-        cudaMemcpyAsync(doff, stream_offsets, (size_t)(R + 1) * 8, cudaMemcpyHostToDevice, h->stream);
-        ga.ustream = dstream;
-        ga.uoff = doff;
-        ga.uused = dused;
-    }
     int wpc = 4;
     int grid = (R + wpc - 1) / wpc;
     int maxgrid = h->num_sms * 16;
     if (grid > maxgrid) grid = maxgrid;
     genealogy_kernel<<<grid, wpc * 32, 0, h->stream>>>(h->st, ga);
     h->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    gfree(h, dseeds);
-    gfree(h, dstream);
-    gfree(h, doff);
-    gfree(h, dused);
-    if (e != cudaSuccess) {
-        cudaFree(I_saved);
-        return vgsim_set_error(cudaGetErrorString(e));
-    }
-    // side-table overflow?  clear the bit and go round again with larger tables
+    CK(cudaGetLastError());
     std::vector<int> errs(R);
-    cudaMemcpy(errs.data(), h->st.err, (size_t)R * 4, cudaMemcpyDeviceToHost);
-    bool overflow = false;
+    CK(cudaMemcpyAsync(errs.data(), h->st.err, (size_t)R * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    *overflow = false;
     for (int &v : errs)
         if (v & ERR_SIDE_TABLE) {
-            overflow = true;
+            *overflow = true;
             v &= ~ERR_SIDE_TABLE;
         }
-    if (!overflow) break;
-    cudaMemcpy(h->st.err, errs.data(), (size_t)R * 4, cudaMemcpyHostToDevice);
-    if (attempt >= 3) {
-        cudaFree(I_saved);
-        return vgsim_set_error("genealogy side tables overflow even at 512x the default capacity");
+    if (*overflow) {
+        CK(cudaMemcpyAsync(h->st.err, errs.data(), (size_t)R * 4, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
     }
-    }
-    cudaFree(I_saved);
-    GenealogyBuffers &G = h->gen;
-    G.valid = true;
     return 0;
 }
 
-static int gen_counts(vgsim_handle h, int r, int *nodes, int *muts, int *migs) {
-    if (!h->gen.valid || r < 0 || r >= h->R) return 1;
-    cudaSetDevice(h->device);
-    if (nodes) cudaMemcpy(nodes, h->gen.n_nodes + r, 4, cudaMemcpyDeviceToHost);
-    if (muts) cudaMemcpy(muts, h->gen.mut_n + r, 4, cudaMemcpyDeviceToHost);
-    if (migs) cudaMemcpy(migs, h->gen.mig_n + r, 4, cudaMemcpyDeviceToHost);
+// *n = counts[r] of one of the genealogy's per-replicate counts (n_nodes, mut_n, mig_n)
+int gen_count(Handle *h, int r, const int *counts, int *n) {
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(n, counts + r, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int vgsim_genealogy(vgsim_handle h, const uint64_t *seeds, const double *uniform_stream, const int64_t *stream_offsets,
+                    int raw_words) {
+    CK(cudaSetDevice(h->device));
+    if (!h->st.first_simulation) return fail("nothing was simulated");
+    if (uniform_stream && !stream_offsets) return fail("stream_offsets is required with uniform_stream");
+    const int R = h->R;
+    std::vector<long long> ctr((size_t)R * NCOUNT);
+    CK(cudaMemcpyAsync(ctr.data(), h->st.counters, ctr.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    GenArgs ga{};
+    ga.raw_words = raw_words;
+    Scratch<unsigned long long> dseeds;
+    Scratch<double> dstream;
+    Scratch<long long> doff, dused;
+    if (seeds) {
+        if (dseeds.alloc(R)) return 1;
+        CK(cudaMemcpyAsync(dseeds, seeds, (size_t)R * 8, cudaMemcpyHostToDevice, h->stream));
+        ga.new_seeds = dseeds;
+    }
+    if (uniform_stream) {
+        const long long n = stream_offsets[R];
+        if (dstream.alloc(n) || doff.alloc(R + 1) || dused.alloc(R)) return 1;
+        CK(cudaMemcpyAsync(dstream, uniform_stream, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(doff, stream_offsets, (size_t)(R + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+        ga.ustream = dstream;
+        ga.uoff = doff;
+        ga.uused = dused;
+    }
+    // The mutation / migration side tables grow with rate x branch length, not with the sample count (the reference
+    // appends to std::vectors, src/models.pxi): start from a size that covers the usual case and, if a replicate
+    // overflows, run the replay again with 8x larger tables.  The replay rewinds the infectious counts in place (quirk
+    // Q9), so they are saved first and put back before a retry.
+    const size_t I_n = (size_t)R * h->D.K * h->D.H;
+    Scratch<long long> I_saved;
+    if (I_saved.alloc(I_n)) return 1;
+    CK(cudaMemcpyAsync(I_saved, h->st.I, I_n * 8, cudaMemcpyDeviceToDevice, h->stream));
+    for (long long attempt = 0, table_scale = 1;; attempt++, table_scale *= 8) {
+        if (attempt > 0) CK(cudaMemcpyAsync(h->st.I, I_saved, I_n * 8, cudaMemcpyDeviceToDevice, h->stream));
+        bool overflow = false;
+        if (replay(h, ctr, table_scale, ga, &overflow)) return 1;
+        if (!overflow) break;
+        if (attempt >= 3) return fail("genealogy side tables overflow even at 512x the default capacity");
+    }
+    h->gen.valid = true;
     return 0;
 }
 
 int64_t vgsim_tree_size(vgsim_handle h, int r) {
-    if (!h->gen.valid || r < 0 || r >= h->R) return 0;
+    if (check_replicate(h, r)) return -1;
+    if (!h->gen.valid) return 0;
     return h->gen.h_node_off[r + 1] - h->gen.h_node_off[r];
 }
 
 int vgsim_get_tree(vgsim_handle h, int r, int64_t *parent, int64_t *pop, double *time) {
-    if (!h->gen.valid) return vgsim_set_error("genealogy was not simulated");
-    if (r < 0 || r >= h->R) return vgsim_set_error("replicate out of range");
-    cudaSetDevice(h->device);
-    long long n = h->gen.h_node_off[r + 1] - h->gen.h_node_off[r], off = h->gen.h_node_off[r];
-    std::vector<int> a(n), b(n);
-    cudaMemcpy(a.data(), h->gen.parent + off, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(b.data(), h->gen.pop + off, n * 4, cudaMemcpyDeviceToHost);
-    if (time) cudaMemcpy(time, h->gen.time + off, n * 8, cudaMemcpyDeviceToHost);
+    if (!h->gen.valid) return fail("genealogy was not simulated");
+    if (check_replicate(h, r)) return 1;
+    const long long n = h->gen.h_node_off[r + 1] - h->gen.h_node_off[r], off = h->gen.h_node_off[r];
+    if (n == 0) return 0;
     int used = 0;
-    gen_counts(h, r, &used, nullptr, nullptr);
+    if (gen_count(h, r, h->gen.n_nodes, &used)) return 1;
+    std::vector<int> a(n), b(n);
+    CK(cudaMemcpyAsync(a.data(), h->gen.parent + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(b.data(), h->gen.pop + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (time) CK(cudaMemcpyAsync(time, h->gen.time + off, n * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     for (long long i = 0; i < n; i++) {
         // nodes never created (incomplete coalescence) read as the reference's zero-initialised arrays
         if (parent) parent[i] = i < used ? a[i] : 0;
@@ -738,19 +712,22 @@ int vgsim_get_tree(vgsim_handle h, int r, int64_t *parent, int64_t *pop, double 
 
 int64_t vgsim_num_mutations(vgsim_handle h, int r) {
     int n = 0;
-    if (gen_counts(h, r, nullptr, &n, nullptr)) return 0;
+    if (check_replicate(h, r) || (h->gen.valid && gen_count(h, r, h->gen.mut_n, &n))) return -1;
     return n;
 }
 
 int vgsim_get_mutations(vgsim_handle h, int r, int64_t *node, int64_t *AS, int64_t *DS, int64_t *site, double *time) {
-    if (!h->gen.valid) return vgsim_set_error("genealogy was not simulated");
-    int n = (int)vgsim_num_mutations(h, r);
+    if (!h->gen.valid) return fail("genealogy was not simulated");
+    int n = 0;
+    if (check_replicate(h, r) || gen_count(h, r, h->gen.mut_n, &n)) return 1;
+    if (n == 0) return 0;
     long long off = h->gen.h_mut_off[r];
     std::vector<int> a(n), b(n), c(n);
-    cudaMemcpy(a.data(), h->gen.mut_node + off, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(b.data(), h->gen.mut_hap + off, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(c.data(), h->gen.mut_nhap + off, n * 4, cudaMemcpyDeviceToHost);
-    if (time) cudaMemcpy(time, h->gen.mut_time + off, n * 8, cudaMemcpyDeviceToHost);
+    CK(cudaMemcpyAsync(a.data(), h->gen.mut_node + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(b.data(), h->gen.mut_hap + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(c.data(), h->gen.mut_nhap + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (time) CK(cudaMemcpyAsync(time, h->gen.mut_time + off, n * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     for (int i = 0; i < n; i++) {
         // Mutations.AddMutation (src/models.pxi:12-26): site counted from the least-significant base-4 digit
         long long x = std::llabs((long long)c[i] - b[i]), s = 0;
@@ -770,19 +747,22 @@ int vgsim_get_mutations(vgsim_handle h, int r, int64_t *node, int64_t *AS, int64
 
 int64_t vgsim_num_migrations(vgsim_handle h, int r) {
     int n = 0;
-    if (gen_counts(h, r, nullptr, nullptr, &n)) return 0;
+    if (check_replicate(h, r) || (h->gen.valid && gen_count(h, r, h->gen.mig_n, &n))) return -1;
     return n;
 }
 
 int vgsim_get_migrations(vgsim_handle h, int r, int64_t *node, double *time, int64_t *old_pop, int64_t *new_pop) {
-    if (!h->gen.valid) return vgsim_set_error("genealogy was not simulated");
-    int n = (int)vgsim_num_migrations(h, r);
+    if (!h->gen.valid) return fail("genealogy was not simulated");
+    int n = 0;
+    if (check_replicate(h, r) || gen_count(h, r, h->gen.mig_n, &n)) return 1;
+    if (n == 0) return 0;
     long long off = h->gen.h_mig_off[r];
     std::vector<int> a(n), b(n), c(n);
-    cudaMemcpy(a.data(), h->gen.mig_node + off, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(b.data(), h->gen.mig_old + off, n * 4, cudaMemcpyDeviceToHost);
-    cudaMemcpy(c.data(), h->gen.mig_new + off, n * 4, cudaMemcpyDeviceToHost);
-    if (time) cudaMemcpy(time, h->gen.mig_time + off, n * 8, cudaMemcpyDeviceToHost);
+    CK(cudaMemcpyAsync(a.data(), h->gen.mig_node + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(b.data(), h->gen.mig_old + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(c.data(), h->gen.mig_new + off, n * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (time) CK(cudaMemcpyAsync(time, h->gen.mig_time + off, n * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     for (int i = 0; i < n; i++) {
         if (node) node[i] = a[i];
         if (old_pop) old_pop[i] = b[i];

@@ -3,6 +3,7 @@
 #include <string>
 #include "../../include/vgsim_b200.h"
 #include "common.cuh"
+#include "host.h"
 #include "samplers.cuh"
 #include "genrng.cuh"
 #include "choose.cuh"
@@ -28,16 +29,14 @@ __global__ void poisson_tap_kernel(const double *lam, long long n, uint64_t seed
 }  // namespace vg
 
 extern "C" int vgsim_test_poisson(const double *lam, int64_t n, uint64_t seed, int64_t *out) {
-    double *dl = nullptr;
-    long long *dout = nullptr;
-    if (cudaMalloc(&dl, n * 8) != cudaSuccess || cudaMalloc(&dout, n * 8) != cudaSuccess) return 1;
-    cudaMemcpy(dl, lam, n * 8, cudaMemcpyHostToDevice);
+    vg::Scratch<double> dl;
+    vg::Scratch<long long> dout;
+    if (dl.alloc(n) || dout.alloc(n)) return 1;
+    CK(cudaMemcpy(dl, lam, n * 8, cudaMemcpyHostToDevice));
     vg::poisson_tap_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dl, n, seed, dout);
-    cudaError_t e = cudaDeviceSynchronize();
-    cudaMemcpy(out, dout, n * 8, cudaMemcpyDeviceToHost);
-    cudaFree(dl);
-    cudaFree(dout);
-    return e == cudaSuccess ? 0 : 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(out, dout, n * 8, cudaMemcpyDeviceToHost));
+    return 0;
 }
 
 namespace vg {
@@ -63,23 +62,20 @@ __global__ void hyper_tap_kernel(const long long *good, const long long *bad, co
 // sequential draws from an injected raw-word stream (numpy PCG64 semantics), for draw-for-draw parity
 extern "C" int vgsim_test_hypergeometric(const int64_t *good, const int64_t *bad, const int64_t *sample, int64_t n,
                                          const uint64_t *raw_words, int64_t n_words, int64_t *out, int64_t *words_used) {
-    long long *dg, *db, *ds, *dout, *dused;
-    unsigned long long *dw;
-    if (cudaMalloc(&dg, n * 8) || cudaMalloc(&db, n * 8) || cudaMalloc(&ds, n * 8) || cudaMalloc(&dout, n * 8) ||
-        cudaMalloc(&dused, 8) || cudaMalloc(&dw, n_words * 8))
-        return 1;
-    cudaMemcpy(dg, good, n * 8, cudaMemcpyHostToDevice);
-    cudaMemcpy(db, bad, n * 8, cudaMemcpyHostToDevice);
-    cudaMemcpy(ds, sample, n * 8, cudaMemcpyHostToDevice);
-    cudaMemcpy(dw, raw_words, n_words * 8, cudaMemcpyHostToDevice);
+    vg::Scratch<long long> dg, db, ds, dout, dused;
+    vg::Scratch<unsigned long long> dw;
+    if (dg.alloc(n) || db.alloc(n) || ds.alloc(n) || dout.alloc(n) || dused.alloc(1) || dw.alloc(n_words)) return 1;
+    CK(cudaMemcpy(dg, good, n * 8, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(db, bad, n * 8, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(ds, sample, n * 8, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dw, raw_words, n_words * 8, cudaMemcpyHostToDevice));
     vg::hyper_tap_kernel<<<1, 32>>>(dg, db, ds, n, dw, n_words, dout, dused);
-    cudaError_t e = cudaDeviceSynchronize();
-    cudaMemcpy(out, dout, n * 8, cudaMemcpyDeviceToHost);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(out, dout, n * 8, cudaMemcpyDeviceToHost));
     long long u = 0;
-    cudaMemcpy(&u, dused, 8, cudaMemcpyDeviceToHost);
+    CK(cudaMemcpy(&u, dused, 8, cudaMemcpyDeviceToHost));
     if (words_used) *words_used = u;
-    cudaFree(dg); cudaFree(db); cudaFree(ds); cudaFree(dout); cudaFree(dused); cudaFree(dw);
-    return e == cudaSuccess ? 0 : 1;
+    return 0;
 }
 
 // ---- cumulative search tap (choose.cuh): one warp per query
@@ -101,20 +97,16 @@ __global__ void choose_tap_kernel(const double *w, int n, const double *x, int m
 
 extern "C" int vgsim_test_choose(const double *w, int n, const double *x, int m, int skip, int small, int64_t *idx,
                                  double *before, double *wsel, double *resid) {
-    double *dw = nullptr, *dx = nullptr, *db = nullptr, *dws = nullptr, *dr = nullptr;
-    long long *di = nullptr;
-    if (cudaMalloc(&dw, (size_t)(n > 0 ? n : 1) * 8) != cudaSuccess || cudaMalloc(&dx, (size_t)m * 8) != cudaSuccess ||
-        cudaMalloc(&db, (size_t)m * 8) != cudaSuccess || cudaMalloc(&dws, (size_t)m * 8) != cudaSuccess ||
-        cudaMalloc(&dr, (size_t)m * 8) != cudaSuccess || cudaMalloc(&di, (size_t)m * 8) != cudaSuccess)
-        return 1;
-    cudaMemcpy(dw, w, (size_t)n * 8, cudaMemcpyHostToDevice);
-    cudaMemcpy(dx, x, (size_t)m * 8, cudaMemcpyHostToDevice);
+    vg::Scratch<double> dw, dx, db, dws, dr;
+    vg::Scratch<long long> di;
+    if (dw.alloc(n) || dx.alloc(m) || db.alloc(m) || dws.alloc(m) || dr.alloc(m) || di.alloc(m)) return 1;
+    CK(cudaMemcpy(dw, w, (size_t)n * 8, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dx, x, (size_t)m * 8, cudaMemcpyHostToDevice));
     vg::choose_tap_kernel<<<(m + 3) / 4, 128>>>(dw, n, dx, m, skip, small, di, db, dws, dr);
-    cudaError_t e = cudaDeviceSynchronize();
-    cudaMemcpy(idx, di, (size_t)m * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(before, db, (size_t)m * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(wsel, dws, (size_t)m * 8, cudaMemcpyDeviceToHost);
-    cudaMemcpy(resid, dr, (size_t)m * 8, cudaMemcpyDeviceToHost);
-    cudaFree(dw); cudaFree(dx); cudaFree(db); cudaFree(dws); cudaFree(dr); cudaFree(di);
-    return e == cudaSuccess ? 0 : 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(idx, di, (size_t)m * 8, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(before, db, (size_t)m * 8, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(wsel, dws, (size_t)m * 8, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(resid, dr, (size_t)m * 8, cudaMemcpyDeviceToHost));
+    return 0;
 }
