@@ -122,7 +122,12 @@ int vgsim_archive_stats(vgsim_handle h, int64_t *entries_total, int64_t *entries
 
 /* SimulatePopulation (src/_BirthDeath.pyx:396-429): batched direct Gillespie, one warp per
  * replicate.  `epidemic_time` is a C float like the reference's (quirk Q1); -1 = no limit;
- * sample_size -1 = no limit.  Appends up to `iterations` rows to each replicate's event log. */
+ * sample_size -1 = no limit.  Appends up to `iterations` rows to each replicate's event log.
+ * Every shape vgsim_create accepts runs: a shape whose rate hierarchy fits one SM's shared memory runs on the
+ * shared-memory kernel, any other on the large-state kernel, which keeps each replicate's rates in 32-ary sum trees in
+ * device memory (one slice per resident warp, allocated at its first call and held by the handle, at most half of the
+ * free device memory).  The two kernels draw from independent streams: they agree in distribution, not draw for draw.
+ * vgsim_set_direct_variant bit 0 runs the large-state kernel on every shape. */
 int vgsim_simulate_direct(vgsim_handle h, int64_t iterations, int64_t sample_size, float epidemic_time,
                           int64_t attempts);
 /* SimulatePopulation_tau (src/_BirthDeath.pyx:2293-2346): replicate-batched tau-leaping, one CTA
@@ -150,7 +155,10 @@ int64_t vgsim_prop_num(vgsim_handle h);
 int vgsim_propensities(vgsim_handle h, int replicate, double *out, double *dI, double *dS, double *tau);
 /* vgsim_rates = the direct-method rate hierarchy after UpdateAllRates (:279-351) computed by the
  * direct kernel's device code: actual sizes A[K], eff[K][K], maxEBM[K], event rates ev[K][H][4],
- * hapPopRate[K][H], popRate[K], migPopRate[K], totals[2] = {totalRate, totalMigrationRate}. */
+ * hapPopRate[K][H], popRate[K], migPopRate[K], totals[2] = {totalRate, totalMigrationRate}.  On shapes that
+ * vgsim_simulate_direct runs on the large-state kernel (and on every shape with vgsim_set_direct_variant bit 0) the
+ * numbers come from that kernel's sum trees: hapPopRate[p,h] = c[p] sum_s Sx[p,s] b[h] sigma[s,h] I[p,h] + (d[h] +
+ * sr[h] sm[p] + tm[h]) I[p,h], popRate and totalRate from the deme tree. */
 int vgsim_rates(vgsim_handle h, int replicate, double *A, double *eff, double *maxEBM, double *ev,
                 double *hapPopRate, double *popRate, double *migPopRate, double *totals);
 
@@ -218,7 +226,9 @@ int vgsim_summaries_dev(vgsim_handle h, void **dev_ptr);
  *   reference's Data / Sample arrays mix these in through an operator-precedence quirk; the Python wrapper rebuilds
  *   its exact output from them);
  *   last_point[rep_count] : index of the grid point that holds the last log row (the reference leaves later points
- *   zero, here they repeat the final state). */
+ *   zero, here they repeat the final state).
+ * A replicate whose counts do not fit one SM's shared memory is replayed in a device scratch slice instead (one per
+ * resident warp, freed on return, at most half of the free device memory); the results are the same. */
 int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step_num, int64_t *infectious,
                           int64_t *susceptible, int64_t *removed, int64_t *sampled, double *time_points,
                           int32_t *last_point);
@@ -234,6 +244,10 @@ int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step
  * forces the former, bit 3 the latter.  Bits 4 and 5 switch off the warp kernel's lockstep generations and its
  * size-sorted replicate schedule (scheduling only as well; tests check that the log does not change). */
 int vgsim_set_tau_variant(vgsim_handle h, int variant);
+/* Parity tap of the direct method.  Bit 0: vgsim_simulate_direct and vgsim_rates use the large-state kernel (sum
+ * trees in device memory) on every shape, not only on shapes whose rate hierarchy exceeds one SM's shared memory.
+ * Default 0.  Tests compare the two kernels in distribution and the trees with the reference's rates. */
+int vgsim_set_direct_variant(vgsim_handle h, int variant);
 /* Measurement tap: with bit 1 of the variant set, thread 0 of every CTA of the tau kernel accumulates the clock
  * cycles between consecutive barriers of the leap loop (critical path per phase: 0 row wipe + lists + Q,
  * 1 drifts + tau, 2 primary draws, 3 slow-path drain, 4 feasibility, 5 apply, 6 lockdown vote, 7 = #leaps)

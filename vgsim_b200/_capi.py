@@ -28,7 +28,7 @@ def _load():
         # in-tree build (nvcc cross-compiles sm_100a without a GPU); raises if nvcc is unavailable
         _build.build()
     lib = ctypes.CDLL(LIB_PATH)
-    if not hasattr(lib, "vgsim_recycle_log") and LIB_PATH == _build.LIB and _build.have_nvcc():
+    if not hasattr(lib, "vgsim_set_direct_variant") and LIB_PATH == _build.LIB and _build.have_nvcc():
         # a library built from older sources (it lacks the newest entry point): rebuild once and load the new file
         del lib
         _build.build(force=True)
@@ -79,6 +79,7 @@ def _load():
         "vgsim_summaries_dev": (c_int, [P, ctypes.POINTER(c_void_p)]),
         "vgsim_launch_count": (c_int64, [P]),
         "vgsim_set_tau_variant": (c_int, [P, c_int]),
+        "vgsim_set_direct_variant": (c_int, [P, c_int]),
         "vgsim_debug_tau_phases": (c_int, [P, P, c_int]),
         "vgsim_debug_tau_cta_end": (c_int, [P, P, c_int]),
         "vgsim_last_kernel_ms": (c_int, [P, ctypes.POINTER(c_float)]),
@@ -422,6 +423,11 @@ class Handle:
         """0 = small mutation / out-migration groups drawn as one Poisson total + multinomial split (product path),
         1 = every channel drawn separately like the reference (parity tap)."""
         _ck(lib.vgsim_set_tau_variant(self._h, int(variant)))
+
+    def set_direct_variant(self, variant):
+        """0 = the shared-memory direct kernel wherever a replicate's rates fit one SM's shared memory, the large-state
+        kernel elsewhere; bit 0 = the large-state kernel on every shape (parity tap)."""
+        _ck(lib.vgsim_set_direct_variant(self._h, int(variant)))
 
 
 def test_poisson(lam, seed=1):

@@ -497,6 +497,50 @@ static SimArgs make_args(int64_t iterations, int64_t sample_size, float t, int64
     return a;
 }
 
+// the parameter point every replicate uses, or -1 when they differ
+static int uniform_pp(const Handle *h) {
+    int u = h->rep_pp_host.empty() ? 0 : h->rep_pp_host[0];
+    for (int v : h->rep_pp_host)
+        if (v != u) u = -1;
+    return u;
+}
+
+static int check_tau_shape(const Handle *h) {
+    if (tau_fits(h->D, uniform_pp(h))) return 0;
+    const Dims &D = h->D;
+    return fail("tau-leaping: one replicate of this shape (" + std::to_string(D.U) + " sites = " + std::to_string(D.H) +
+                " haplotypes, " + std::to_string(D.K) + " demes, " + std::to_string(D.S) +
+                " susceptibility groups) exceeds one SM's shared memory, which the tau kernels need; simulate this shape "
+                "with the direct method (vgsim_simulate_direct)");
+}
+
+// Warp slices of the large-state direct kernel: one per resident warp (at most 16 per SM) that the batch can use, capped
+// so that they take at most half of the device memory that is free (the slices already held count as free).  Grown,
+// never shrunk.  nwarps: slices available.
+static int dl_slices(Handle *h, const DLLayout &L, int &nwarps) {
+    size_t fr = 0, tot = 0;
+    CK(cudaMemGetInfo(&fr, &tot));
+    const size_t slice = (size_t)L.slice * 8;
+    const size_t fit = (fr / 2 + h->dl_slices_n * 8) / slice;
+    size_t nw = std::min<size_t>(std::min<size_t>(h->R, (size_t)h->num_sms * 16), fit);
+    if (nw < 1)
+        return fail("direct kernel: one replicate's state (" + std::to_string(slice >> 20) +
+                    " MB of rate trees) exceeds half of the free device memory");
+    if (h->dl_slices_n < nw * L.slice) {
+        dfree(h, h->dl_slices);
+        h->dl_slices = nullptr;
+        h->dl_slices_n = 0;
+        if (dalloc(h, &h->dl_slices, nw * L.slice)) return 1;
+        h->dl_slices_n = nw * L.slice;
+    }
+    nwarps = (int)(h->dl_slices_n / L.slice < nw ? h->dl_slices_n / L.slice : nw);
+    return 0;
+}
+
+// the large-state direct kernel runs the shapes whose rate hierarchy does not fit the shared-memory kernel, and every
+// shape with vgsim_set_direct_variant bit 0
+static bool direct_large(const Handle *h, int upp) { return (h->direct_variant & 1) || !direct_fits_shared(h->D, upp); }
+
 extern "C" {
 
 // one launch of the tau kernel for `iterations` more leaps per replicate.  tau_mode 1: a call of SimulatePopulation_tau
@@ -513,10 +557,7 @@ static int tau_call(Handle *h, int64_t iterations, int64_t sample_size, float ep
         next_timer(h);
         CK(cudaEventRecord(h->ev_k0, h->stream));
     }
-    int uniform_pp = h->rep_pp_host.empty() ? 0 : h->rep_pp_host[0];  // every replicate on one parameter point?
-    for (int v : h->rep_pp_host)
-        if (v != uniform_pp) uniform_pp = -1;
-    cudaError_t e = launch_tau(h->st, a, h->stream, h->num_sms, h->tau_variant, uniform_pp, h->tau_order);
+    cudaError_t e = launch_tau(h->st, a, h->stream, h->num_sms, h->tau_variant, uniform_pp(h), h->tau_order);
     if (e != cudaSuccess) return fail(std::string("tau kernel: ") + cudaGetErrorString(e));
     if (timed) {
         CK(cudaEventRecord(h->ev_k1, h->stream));
@@ -533,6 +574,7 @@ int vgsim_simulate_tau(vgsim_handle h, int64_t iterations, int64_t sample_size, 
                        int64_t attempts) {
     CK(cudaSetDevice(h->device));
     if (iterations < 0) return fail("iterations must be >= 0");
+    if (check_tau_shape(h)) return 1;
     return tau_call(h, iterations, sample_size, epidemic_time, attempts, 1, true);
 }
 
@@ -546,6 +588,7 @@ int vgsim_simulate_tau_blocks(vgsim_handle h, int64_t iterations, int64_t sample
     CK(cudaSetDevice(h->device));
     if (iterations < 0) return fail("iterations must be >= 0");
     if (leap_block < 1) return fail("leap_block must be >= 1");
+    if (check_tau_shape(h)) return 1;
     // the extinction retry looks at the call's `iterations > 100` (:2331): a block must not hide that from the kernel
     if (iterations > 100 && leap_block <= 100) leap_block = 101;
     next_timer(h);
@@ -645,12 +688,15 @@ int vgsim_simulate_direct(vgsim_handle h, int64_t iterations, int64_t sample_siz
     if (ensure_ev_cap(h, h->ev_bound + iterations)) return 1;
     if (prepare(h, 0)) return 1;
     SimArgs a = make_args(iterations, sample_size, epidemic_time, attempts);
+    const int upp = uniform_pp(h);
+    const bool large = direct_large(h, upp);
+    const DLLayout L = dl_layout(h->D);
+    int nwarps = 0;
+    if (large && dl_slices(h, L, nwarps)) return 1;
     next_timer(h);
     CK(cudaEventRecord(h->ev_k0, h->stream));
-    int uniform_pp = h->rep_pp_host.empty() ? 0 : h->rep_pp_host[0];  // every replicate on one parameter point?
-    for (int v : h->rep_pp_host)
-        if (v != uniform_pp) uniform_pp = -1;
-    cudaError_t e = launch_direct(h->st, a, h->stream, h->num_sms, uniform_pp, h->work);
+    cudaError_t e = large ? launch_direct_large(h->st, a, L, h->dl_slices, nwarps, h->num_sms, h->stream, h->work)
+                          : launch_direct(h->st, a, h->stream, h->num_sms, upp, h->work);
     if (e != cudaSuccess) return fail(std::string("direct kernel: ") + cudaGetErrorString(e));
     CK(cudaEventRecord(h->ev_k1, h->stream));
     h->ev_valid = true;
@@ -691,6 +737,7 @@ int vgsim_propensities(vgsim_handle h, int replicate, double *out, double *dI, d
     CK(cudaSetDevice(h->device));
     if (check_replicate(h, replicate)) return 1;
     if (!h->hp[0].uploaded) return fail("parameters were not uploaded");
+    if (check_tau_shape(h)) return 1;
     const Dims &D = h->D;
     // like PrintPropensities: UpdateAllRates on the CURRENT state (no FirstInfection, no lockdown check)
     cudaError_t e = launch_refresh(h->st, h->stream);
@@ -723,8 +770,16 @@ int vgsim_rates(vgsim_handle h, int replicate, double *A, double *eff, double *m
     size_t n = (size_t)K * H * 4 + (size_t)K * H + K + K + 2;
     Scratch<double> buf;
     if (buf.alloc(n)) return 1;
-    e = launch_rates_tap(h->st, replicate, buf, buf + K * H * 4, buf + K * H * 5, buf + K * H * 5 + K,
-                         buf + K * H * 5 + 2 * K, h->stream);
+    Scratch<double> slice;
+    if (direct_large(h, -1)) {  // the large-state kernel's trees, built as that kernel builds them
+        const DLLayout L = dl_layout(D);
+        if (slice.alloc(L.slice)) return 1;
+        e = launch_rates_large(h->st, L, slice, replicate, buf, buf + K * H * 4, buf + K * H * 5, buf + K * H * 5 + K,
+                               buf + K * H * 5 + 2 * K, h->stream);
+    } else {
+        e = launch_rates_tap(h->st, replicate, buf, buf + K * H * 4, buf + K * H * 5, buf + K * H * 5 + K,
+                             buf + K * H * 5 + 2 * K, h->stream);
+    }
     h->launches += 2;
     if (e != cudaSuccess) return fail(std::string("rates kernel: ") + cudaGetErrorString(e));
     std::vector<double> hb(n);
@@ -916,10 +971,24 @@ int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step
     if ((infectious && d_inf.alloc(np * KH)) || (susceptible && d_sus.alloc(np * KS)) || (removed && d_rem.alloc(np * KH)) ||
         (sampled && d_smp.alloc(np * KH)) || (time_points && d_tp.alloc(np)) || (last_point && d_lp.alloc(rep_count)))
         return 1;
+    // replicates whose counts do not fit one SM's shared memory replay in device slices: one per resident warp (at most
+    // 16 per SM), at most half of the free device memory
+    const bool tallies = removed || sampled;
+    Scratch<unsigned char> d_slices;
+    int nslices = 0;
+    if (!curves_fit_shared(D, tallies)) {
+        size_t fr = 0, tot = 0;
+        CK(cudaMemGetInfo(&fr, &tot));
+        const size_t sb = curves_slice_bytes(D, tallies);
+        const size_t nw = std::min<size_t>(std::min<size_t>(rep_count, (size_t)h->num_sms * 16), fr / 2 / sb);
+        if (nw < 1) return fail("epidemic curves: one replicate's counts exceed half of the free device memory");
+        if (d_slices.alloc(nw * sb)) return 1;
+        nslices = (int)nw;
+    }
     next_timer(h);
     CK(cudaEventRecord(h->ev_k0, h->stream));  // vgsim_last_kernel_ms then reports this kernel
     cudaError_t e = launch_curves(h->st, rep_first, rep_count, step_num, d_inf, d_sus, d_rem, d_smp, d_tp, d_lp, h->stream,
-                                  h->num_sms);
+                                  h->num_sms, d_slices, nslices);
     CK(cudaEventRecord(h->ev_k1, h->stream));
     h->ev_valid = true;
     h->launches++;
@@ -954,6 +1023,12 @@ int vgsim_set_tau_variant(vgsim_handle h, int variant) {
     if (variant < 0 || variant > 63 || (variant & 12) == 12)
         return fail("tau variant must be 0..63 (bit 0: per-channel draws, bit 1: phase timing, bit 2: force the team kernel, bit 3: force the warp kernel, bit 4: free-running warps, bit 5: unsorted schedule)");
     h->tau_variant = variant;
+    return 0;
+}
+
+int vgsim_set_direct_variant(vgsim_handle h, int variant) {
+    if (variant < 0 || variant > 1) return fail("direct variant must be 0 or 1 (bit 0: the large-state kernel on every shape)");
+    h->direct_variant = variant;
     return 0;
 }
 

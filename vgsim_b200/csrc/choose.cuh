@@ -29,6 +29,13 @@ struct Pick {
     }
 };
 
+// sum over the lanes of a warp, every lane gets it; a butterfly, so the result is the same function of the 32 lane
+// values in every lane and every call
+__device__ __forceinline__ double warp_sum(double v) {
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
 // inclusive prefix sum over the lanes of a warp; lanes >= n must hold 0 (steps beyond n are skipped)
 __device__ __forceinline__ double warp_scan_incl(double v, int n) {
     const int lane = threadIdx.x & 31;

@@ -66,11 +66,15 @@ __device__ __forceinline__ void curve_apply(int type, int hap, int pop, int nhap
     }
 }
 
-__global__ void __launch_bounds__(512, 1) curves_kernel(const DevState st, const CurveArgs a, int slice_bytes) {
+// The replay; GSLICE: the warps' slices live in gslices (one per warp of the grid, curves_large_kernel: replicates whose
+// counts do not fit one SM's shared memory), else in shared memory (curves_kernel).
+template <bool GSLICE>
+__device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs &a, int slice_bytes, unsigned char *gslices) {
     const Dims &D = st.D;
     const int K = D.K, H = D.H, S = D.S, KH = K * H, KS = K * S;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    unsigned long long *I = reinterpret_cast<unsigned long long *>(curves_smem + (size_t)wid * slice_bytes);
+    unsigned long long *I = reinterpret_cast<unsigned long long *>(
+        GSLICE ? gslices + (size_t)(blockIdx.x * nw + wid) * slice_bytes : curves_smem + (size_t)wid * slice_bytes);
     const bool tallies = a.removed != nullptr || a.sampled != nullptr;
     unsigned long long *Sx = I + KH, *rem = tallies ? Sx + KS : nullptr, *smp = tallies ? rem + KH : nullptr;
     // (channel, count) of the non-zero counts of the row being scanned
@@ -232,17 +236,41 @@ __global__ void __launch_bounds__(512, 1) curves_kernel(const DevState st, const
     }
 }
 
+__global__ void __launch_bounds__(512, 1) curves_kernel(const DevState st, const CurveArgs a, int slice_bytes) {
+    curves_body<false>(st, a, slice_bytes, nullptr);
+}
+
+__global__ void __launch_bounds__(512, 1) curves_large_kernel(const DevState st, const CurveArgs a, int slice_bytes,
+                                                               unsigned char *gslices) {
+    curves_body<true>(st, a, slice_bytes, gslices);
+}
+
+size_t curves_slice_bytes(const Dims &D, bool tallies) {
+    const size_t ncell = tallies ? 3 : 1;  // I (+ removed, sampled) per infectious cell
+    return ((ncell * D.K * D.H + (size_t)D.K * D.S) * 8 + CURVE_QCAP * 8 + 15) & ~(size_t)15;
+}
+
+bool curves_fit_shared(const Dims &D, bool tallies) { return curves_slice_bytes(D, tallies) <= 227 * 1024; }
+
 cudaError_t launch_curves(const DevState &st, int rep_first, int rep_count, int step_num, long long *inf, long long *sus,
                           long long *removed, long long *sampled, double *time_points, int *last_point,
-                          cudaStream_t stream, int num_sms) {
+                          cudaStream_t stream, int num_sms, unsigned char *gslices, int nslices) {
     CurveArgs a;
     a.rep_first = rep_first; a.rep_count = rep_count; a.step_num = step_num;
     a.inf = inf; a.sus = sus; a.removed = removed; a.sampled = sampled;
     a.time_points = time_points; a.last_point = last_point;
-    const int ncell = (removed || sampled) ? 3 : 1;  // I (+ removed, sampled) per infectious cell
-    const int slice = ((ncell * st.D.K * st.D.H + st.D.K * st.D.S) * 8 + CURVE_QCAP * 8 + 15) & ~15;
+    const bool tallies = removed || sampled;
+    if (!curves_fit_shared(st.D, tallies)) {  // the state of one replicate does not fit one SM's shared memory
+        if (!gslices || nslices < 1) return cudaErrorInvalidValue;
+        int nw = (nslices + num_sms - 1) / num_sms;  // spread over the SMs, at most 16 warps per CTA
+        if (nw > 16) nw = 16;
+        int grid = nslices / nw;
+        if (grid > (rep_count + nw - 1) / nw) grid = (rep_count + nw - 1) / nw;
+        curves_large_kernel<<<grid, nw * 32, 0, stream>>>(st, a, (int)curves_slice_bytes(st.D, tallies), gslices);
+        return cudaGetLastError();
+    }
+    const int slice = (int)curves_slice_bytes(st.D, tallies);
     int nw = (227 * 1024) / slice;
-    if (nw < 1) return cudaErrorInvalidValue;  // the state of one replicate does not fit one SM's shared memory
     if (nw > 16) nw = 16;
     cudaError_t e = cudaFuncSetAttribute(curves_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, nw * slice);
     if (e != cudaSuccess) return e;

@@ -124,11 +124,6 @@ __device__ __forceinline__ void dir_load_params(const Dims &D, const DirLayout &
     }
 }
 
-__device__ __forceinline__ double warp_sum(double v) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // Q[p,h] = sum_s Sx[p,s] sigma[s,h]: the susceptible pressure on haplotype h in deme p (inner sum of BirthRate, :382-392)
 // SC: the number of susceptibility groups when it is a compile-time constant (1..4: the loops over groups unroll and
 // their address arithmetic folds), 0: taken from D at run time.
@@ -625,6 +620,12 @@ __global__ void rates_tap_kernel(const __grid_constant__ DevState st, const __gr
         totals[0] = Rt;
         totals[1] = y;
     }
+}
+
+// Does one replicate's rate hierarchy fit one SM's shared memory?  uniform_pp >= 0: with the parameter block shared
+// by the CTA (launch_direct when every replicate uses that point); < 0: in the warp's slice (launch_rates_tap too).
+bool direct_fits_shared(const Dims &D, int uniform_pp) {
+    return dir_layout(D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024, 16).nwarps >= 1;
 }
 
 cudaError_t launch_direct(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int uniform_pp, int *work) {

@@ -49,6 +49,9 @@ struct Handle {
     long long dense_bound = 0;               // ... of leaps whose dense row has not been archived
     long long launches = 0;
     int tau_variant = 0;  // 0 = aggregated small groups (product), 1 = one Poisson draw per channel (parity tap)
+    int direct_variant = 0;  // bit 0: the large-state direct kernel on every shape (parity tap)
+    double *dl_slices = nullptr;  // warp slices of the large-state direct kernel (allocated at its first call)
+    size_t dl_slices_n = 0;       // doubles held
     bool state_set = false;
     bool async_host = false;  // vgsim_set_async: host-buffer copies are enqueued without blocking the calling thread
     GenealogyBuffers gen;
@@ -68,6 +71,23 @@ struct Handle {
     std::vector<void *> allocs;
 };
 
+// 32-ary sum tree of the large-state direct kernel (direct_large_kernel.cu): level l has n[l] nodes at offset off[l]
+// (doubles); size: doubles in all.  Depth 4 holds 2^20 leaves (H <= 4^9, K <= 4096).
+#define TREE32_MAXD 4
+struct Tree32 {
+    int depth, size;
+    int off[TREE32_MAXD], n[TREE32_MAXD];
+};
+// One warp slice of the large-state direct kernel, in doubles: K * nt haplotype trees, the deme tree, the per-deme
+// vectors.
+struct DLLayout {
+    Tree32 th, tk;  // over the H haplotypes of a deme, over the K demes
+    int nt;         // trees per deme: S + 2
+    long long o_dtree, o_tm, o_Sx, o_root, o_totSus, o_imm, o_c, o_cd, o_maxEBM, o_lock, o_zs;
+    long long slice;
+};
+DLLayout dl_layout(const Dims &D);
+
 // kernels' host launchers (defined in the .cu files)
 cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant, int uniform_pp,
                        int *order_buf);
@@ -80,10 +100,20 @@ cudaError_t launch_archive_write(const DevState &st, const int *cnt, const int *
 cudaError_t launch_prepare(const DevState &st, int first, int tau_mode, cudaStream_t stream);
 cudaError_t launch_refresh(const DevState &st, cudaStream_t stream);
 cudaError_t launch_direct(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int uniform_pp, int *work);
+bool direct_fits_shared(const Dims &D, int uniform_pp);
+cudaError_t launch_direct_large(const DevState &st, const SimArgs &a, const DLLayout &L, double *slices, int nwarps,
+                                int num_sms, cudaStream_t stream, int *work);
+// one replicate's curve slice in bytes; when it does not fit one SM's shared memory, launch_curves replays in gslices,
+// a device scratch of nslices >= 1 such slices
+size_t curves_slice_bytes(const Dims &D, bool tallies);
+bool curves_fit_shared(const Dims &D, bool tallies);
 cudaError_t launch_curves(const DevState &st, int rep_first, int rep_count, int step_num, long long *inf, long long *sus,
                           long long *removed, long long *sampled, double *time_points, int *last_point,
-                          cudaStream_t stream, int num_sms);
+                          cudaStream_t stream, int num_sms, unsigned char *gslices, int nslices);
 cudaError_t launch_rates_tap(const DevState &st, int r, double *ev, double *hp, double *popRate, double *migPop,
                              double *totals, cudaStream_t stream);
+cudaError_t launch_rates_large(const DevState &st, const DLLayout &L, double *slice, int r, double *ev, double *hp,
+                               double *popRate, double *migPop, double *totals, cudaStream_t stream);
+bool tau_fits(const Dims &D, int uniform_pp);
 
 }  // namespace vg

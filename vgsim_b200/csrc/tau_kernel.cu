@@ -1282,13 +1282,28 @@ static cudaError_t launch_tau_cfg(const DevState &st, const SimArgs &a, cudaStre
     return cudaGetLastError();
 }
 
+// Can the warp-per-replicate kernel hold the shape in layout L?  Cell ids are held as uint16, a cell's local channels
+// in the 12-bit field of a queue entry.
+static bool tau_warp_fits(const Dims &D, const WarpLayout &L) {
+    return L.nwarps >= 1 && D.K * D.H < 65536 && D.E + (D.K - 1) * D.S < 4000;
+}
+static size_t tau_team_stride(const Dims &D) { return ((size_t)tau_layout(D, false, TAU_TEAM).bytes + 15) & ~(size_t)15; }
+
+// Can any tau kernel hold one replicate of this shape (launch_tau's own test, without the variant bits that force one
+// of the two mappings)?
+bool tau_fits(const Dims &D, int uniform_pp) {
+    if ((long long)D.K * D.H + D.K >= (1 << 20)) return false;
+    if (tau_team_stride(D) + TAU_CTA_TAIL <= (size_t)227 * 1024) return true;
+    return tau_warp_fits(D, warp_layout(D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024));
+}
+
 // Default: the warp-per-replicate kernel (tau_warp.cuh), one CTA per SM with as many warps as the shared memory
 // holds (<= 14).  The team kernel (256-thread teams, CTA-wide generations) stays available as a parity tap:
 // variant bit 2 (vgsim_set_tau_variant); bit 3 forces the warp kernel.
 cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant, int uniform_pp,
                        int *order_buf) {
     if ((long long)st.D.K * st.D.H + st.D.K >= (1 << 20)) return cudaErrorInvalidValue;  // owner id is packed in 20 bits
-    const size_t stride = ((size_t)tau_layout(st.D, false, TAU_TEAM).bytes + 15) & ~(size_t)15;
+    const size_t stride = tau_team_stride(st.D);
     int teams = (int)((227 * 1024 - TAU_CTA_TAIL) / stride);
     if (teams > 4) teams = 4;
     if (teams < 1) teams = 1;
@@ -1302,8 +1317,7 @@ cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream
     if (!team) {
         WarpLayout L = warp_layout(st.D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024);
         L.gsync = (variant & 16) ? 0 : 3;  // lockstep generations: the warps of a CTA meet at leap start and before the draws
-        const int LC = st.D.E + (st.D.K - 1) * st.D.S;     // local channels of a cell: 12-bit field of a queue entry
-        if (L.nwarps >= 1 && st.D.K * st.D.H < 65536 && LC < 4000) {  // cell ids are held as uint16
+        if (tau_warp_fits(st.D, L)) {
             const WS ws = make_ws(L, st.D);
             const bool prof = (variant & 2) != 0, masks = L.use_masks != 0;
             const void *kern = L.has_eff ? (masks ? (prof ? (const void *)tau_warp_kernel<true, true, true> : (const void *)tau_warp_kernel<false, true, true>)
