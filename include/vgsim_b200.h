@@ -80,6 +80,27 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
                         const double *contact_density, const double *cd_before, const double *cd_after,
                         const double *startLD, const double *endLD, const double *sampling_multiplier,
                         const int64_t *sizes, const int32_t *cd_reset_mask);
+/* Parameter grid (sweeps described by their axes): points [dst_pp0, dst_pp0 + n_points) become the points
+ * first_point .. first_point + n_points - 1 of the row-major product of n_axes axes (axis 0 slowest, itertools.product
+ * order), built on the device.  Point pp = (c_0, .., c_{n-1}) is the source arrays of the base point base_pp (which must
+ * have been uploaded) with the patch of value c_a of every axis a written over them, in axis order.  Value j of the
+ * concatenated axes (j = axis_len[0] + .. + axis_len[a-1] + c_a) patches entries patch_idx[patch_off[j] ..
+ * patch_off[j+1]) with patch_val[..]; an index addresses the concatenation of the 16 source arrays of
+ * vgsim_upload_params in its argument order (b, d, s, mRate, hapMutType, sigma, suscType, T, m, contact_density,
+ * cd_before, cd_after, startLD, endLD, sampling_multiplier, sizes; suscType and sizes as fp64).  The diagonal of m is
+ * not read: it is 1 - (row's off-diagonal sum), like vgsim_upload_params computes it.  Each point's blob is the same
+ * bits vgsim_upload_params writes for the same arrays.  Every point is checked first: suscType an integer in [0, S),
+ * sizes an integer in [1, 2^31-1], every row of m with an off-diagonal sum <= 1 and a diagonal > 1e-15 (the two rules of
+ * the reference's migration setters).  A failing point fails the whole call with a message naming its grid index and
+ * the rule; nothing is uploaded then.  Otherwise the live contact density of every replicate mapped to one of the
+ * points is set to that point's contact_density (what a first vgsim_upload_params of the point does).  One stream
+ * synchronisation per call; host cost O(sum axis_len + patches), device work O(n_points). */
+int vgsim_upload_param_grid(vgsim_handle h, int base_pp, int n_axes, const int32_t *axis_len,
+                            const int64_t *patch_off /*[sum axis_len + 1]*/, const int64_t *patch_idx,
+                            const double *patch_val, int64_t first_point, int dst_pp0, int n_points);
+/* Read tap: the device blob of parameter point pp (the derived constants the kernels read; its length follows from the
+ * model shape, see Dims in csrc/common.cuh). */
+int vgsim_get_params(vgsim_handle h, int pp, double *blob_out);
 /* replicate -> parameter point map (default: all 0).  Parameter sweeps (BASELINE config 5).  Before the first simulate
  * call the live contact density of every replicate is (re)seeded from its point's uploaded value, whichever of
  * vgsim_upload_params / vgsim_set_replicate_params comes first; after it the map may still change, but contact

@@ -20,6 +20,17 @@ COUNTER_NAMES = ("bCounter", "dCounter", "sCounter", "mCounter", "iCounter", "mi
 
 c_void_p, c_int, c_int64, c_uint64, c_float, c_char_p = (ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
                                                          ctypes.c_uint64, ctypes.c_float, ctypes.c_char_p)
+# the source arrays of vgsim_upload_params in argument order (keys of BirthDeathModel.param_arrays); a parameter grid's
+# patch indices address their concatenation
+SOURCE_FIELDS = ("b", "d", "s", "mRate", "hapMutType", "sigma", "suscType", "T", "m", "cd", "cdBefore", "cdAfter",
+                 "startLD", "endLD", "sm", "sizes")
+
+
+def blob_len(sites, K, S):
+    """Doubles in one parameter point's device blob (the Dims layout of csrc/common.cuh)."""
+    H, Um = 4 ** sites, max(sites, 1)
+    n = 3 * H + 3 * H * sites + H + S * H + S * S + S + K * K + 7 * K + H + 4 * H * Um + 1 + K
+    return (n + 1) & ~1
 
 
 def _load():
@@ -28,7 +39,7 @@ def _load():
         # in-tree build (nvcc cross-compiles sm_100a without a GPU); raises if nvcc is unavailable
         _build.build()
     lib = ctypes.CDLL(LIB_PATH)
-    if not hasattr(lib, "vgsim_set_direct_variant") and LIB_PATH == _build.LIB and _build.have_nvcc():
+    if not hasattr(lib, "vgsim_upload_param_grid") and LIB_PATH == _build.LIB and _build.have_nvcc():
         # a library built from older sources (it lacks the newest entry point): rebuild once and load the new file
         del lib
         _build.build(force=True)
@@ -42,6 +53,8 @@ def _load():
         "vgsim_set_stream": (c_int, [P, P]),
         "vgsim_set_seeds": (c_int, [P, P]),
         "vgsim_upload_params": (c_int, [P, c_int] + [P] * 17),
+        "vgsim_upload_param_grid": (c_int, [P, c_int, c_int, P, P, P, P, c_int64, c_int, c_int]),
+        "vgsim_get_params": (c_int, [P, c_int, P]),
         "vgsim_set_replicate_params": (c_int, [P, P]),
         "vgsim_set_state": (c_int, [P, P, P]),
         "vgsim_get_state": (c_int, [P, P, P, P, P]),
@@ -165,6 +178,21 @@ class Handle:
             cd_mask = np.full(self.K, 1 if reset_contact_density else 0, dtype=np.int32)
         arrs.append(_arr(cd_mask, np.int32))
         _ck(lib.vgsim_upload_params(self._h, pp, *[_p(x) for x in arrs]))
+
+    def upload_param_grid(self, base_pp, axis_len, patch_off, patch_idx, patch_val, first_point, dst_pp0, n_points):
+        """Points [dst_pp0, dst_pp0 + n_points) = points first_point.. of the row-major product of the axes, built on the
+        device from point base_pp and one patch per axis value (include/vgsim_b200.h: vgsim_upload_param_grid)."""
+        axis_len = _arr(axis_len, np.int32)
+        off, idx, val = _arr(patch_off, np.int64), _arr(patch_idx, np.int64), _arr(patch_val, np.float64)
+        assert off.shape == (int(axis_len.sum()) + 1,) and idx.shape == val.shape == (int(off[-1]),)
+        _ck(lib.vgsim_upload_param_grid(self._h, int(base_pp), len(axis_len), _p(axis_len), _p(off), _p(idx), _p(val),
+                                        int(first_point), int(dst_pp0), int(n_points)))
+
+    def get_params(self, pp):
+        """The device blob of parameter point pp (float64[blob_len])."""
+        out = np.zeros(blob_len(self.sites, self.K, self.S), np.float64)
+        _ck(lib.vgsim_get_params(self._h, int(pp), _p(out)))
+        return out
 
     def set_replicate_params(self, mapping):
         m = _arr(mapping, np.int32)

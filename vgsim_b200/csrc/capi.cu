@@ -10,6 +10,7 @@
 #include "../../include/vgsim_b200.h"
 #include "common.cuh"
 #include "host.h"
+#include "param_blob.cuh"
 
 using namespace vg;
 
@@ -143,6 +144,64 @@ int vgsim_set_replicate_params(vgsim_handle h, const int32_t *map) {
     return 0;
 }
 
+static Src<long long> src_view(const HostParams &P) {
+    Src<long long> v;
+    v.b = P.b.data(), v.d = P.d.data(), v.s = P.s.data(), v.mRate = P.mRate.data(), v.hapMutType = P.hapMutType.data();
+    v.sigma = P.sigma.data(), v.T = P.T.data(), v.m = P.m.data(), v.cd = P.cd.data(), v.cdBefore = P.cdBefore.data();
+    v.cdAfter = P.cdAfter.data(), v.startLD = P.startLD.data(), v.endLD = P.endLD.data(), v.sm = P.sm.data();
+    v.suscType = P.suscType.data(), v.sizes = P.sizes.data();
+    return v;
+}
+
+// The fp64 fields of HostParams in vgsim_upload_params order (nullptr: the int64 fields suscType and sizes).
+static void double_fields(HostParams &P, std::vector<double> *f[NSRC]) {
+    std::vector<double> *t[NSRC] = {&P.b, &P.d, &P.s, &P.mRate, &P.hapMutType, &P.sigma, nullptr, &P.T,
+                                    &P.m, &P.cd, &P.cdBefore, &P.cdAfter, &P.startLD, &P.endLD, &P.sm, nullptr};
+    std::copy(t, t + NSRC, f);
+}
+
+static std::vector<double> flatten(const Dims &D, HostParams &P) {
+    std::vector<double> *f[NSRC];
+    double_fields(P, f);
+    std::vector<double> out;
+    out.reserve(src_off(D, NSRC));
+    for (int k = 0; k < NSRC; k++) {
+        if (f[k])
+            out.insert(out.end(), f[k]->begin(), f[k]->end());
+        else
+            for (long long x : k == F_SUSC ? P.suscType : P.sizes) out.push_back((double)x);
+    }
+    return out;
+}
+
+// Host record of parameter point pp; a grid point's is rebuilt from its grid's base and patches at the first use.
+static HostParams &host_params(Handle *h, int pp) {
+    HostParams &P = h->hp[pp];
+    if (!P.grid) return P;
+    const ParamGrid &g = *P.grid;
+    const Dims &D = h->D;
+    std::vector<double> src(g.base);
+    long long start = 0, stride = 1;
+    for (int len : g.axis_len) stride *= len;
+    for (int len : g.axis_len) {
+        stride /= len;
+        const long long j = start + (P.grid_point / stride) % len;
+        for (long long k = g.off[j]; k < g.off[j + 1]; k++) src[g.idx[k]] = g.val[k];
+        start += len;
+    }
+    std::vector<double> *f[NSRC];
+    double_fields(P, f);
+    for (int k = 0; k < NSRC; k++) {
+        const double *a = src.data() + src_off(D, k), *e = a + src_len(D, k);
+        if (f[k])
+            f[k]->assign(a, e);
+        else
+            (k == F_SUSC ? P.suscType : P.sizes).assign(a, e);
+    }
+    P.grid.reset();
+    return P;
+}
+
 __global__ void set_cd_kernel(DevState st, int pp, const int *mask, const double *cdv) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= st.R * st.D.K) return;
@@ -159,7 +218,7 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
     CK(cudaSetDevice(h->device));
     const Dims &D = h->D;
     const int K = D.K, H = D.H, S = D.S, U = D.U;
-    HostParams &P = h->hp[pp];
+    HostParams &P = host_params(h, pp);
     auto cp = [](std::vector<double> &v, const double *src, size_t n, double dflt) {
         if (src)
             v.assign(src, src + n);
@@ -199,63 +258,13 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
         if (P.sizes[p] <= 0 || P.sizes[p] > 2147483647LL)
             return fail("population sizes must be in [1, 2^31-1] (compartment counts are int32 on the device)");
 
-    // ---- derived constants of UpdateAllRates (reference :279-351), fp64, reference summation order
     std::vector<double> blob(D.blob, 0.0);
-    for (int i = 0; i < H; i++) {
-        blob[D.o_b + i] = P.b[i];
-        blob[D.o_d + i] = P.d[i];
-        blob[D.o_sr + i] = P.s[i];
-        blob[D.o_g + i] = (double)P.suscType[i];
-        double tq = 0.0;
-        for (int u = 0; u < U; u++) {
-            const double *w = &P.hapMutType[((size_t)i * U + u) * 3];
-            blob[D.o_mu + i * U + u] = P.mRate[(size_t)i * U + u];
-            for (int k = 0; k < 3; k++) {
-                double q = P.mRate[(size_t)i * U + u] * w[k] / (w[0] + w[1] + w[2]);  // (:2400-2401)
-                blob[D.o_q + (i * U + u) * 3 + k] = q;
-                blob[D.o_w + (i * U + u) * 3 + k] = w[k];
-                tq += q;
-            }
-        }
-        blob[D.o_tmq + i] = tq;
-        for (int sn = 0; sn < S; sn++) blob[D.o_sigT + sn * H + i] = P.sigma[(size_t)i * S + sn];
-    }
-    for (int s1 = 0; s1 < S; s1++) {
-        double tc = 0;
-        for (int s2 = 0; s2 < S; s2++) {
-            blob[D.o_T + s1 * S + s2] = P.T[(size_t)s1 * S + s2];
-            tc += P.T[(size_t)s1 * S + s2];
-        }
-        blob[D.o_Tc + s1] = tc;
-    }
-    std::vector<double> mm(P.m);
-    std::vector<double> A(K, 0.0);
-    for (int p1 = 0; p1 < K; p1++) {
-        mm[(size_t)p1 * K + p1] = 1.0;
-        A[p1] = 0.0;
-        for (int p2 = 0; p2 < K; p2++) {
-            if (p1 == p2) continue;
-            mm[(size_t)p1 * K + p1] -= mm[(size_t)p1 * K + p2];
-            A[p1] += mm[(size_t)p2 * K + p1] * (double)P.sizes[p2];
-        }
-        A[p1] += mm[(size_t)p1 * K + p1] * (double)P.sizes[p1];
-    }
+    const Src<long long> src = src_view(P);
     double maxB = 0.0;
-    for (int i = 0; i < H; i++)
-        for (int sn = 0; sn < S; sn++)
-            if (P.b[i] * P.sigma[(size_t)i * S + sn] > maxB) maxB = P.b[i] * P.sigma[(size_t)i * S + sn];
+    for (int i = 0; i < H; i++) maxB = std::max(maxB, blob_hap(D, src, blob.data(), i));
+    for (int s1 = 0; s1 < S; s1++) blob_group(D, src, blob.data(), s1);
+    for (int p = 0; p < K; p++) blob_deme(D, src, blob.data(), p);
     blob[D.o_maxB] = maxB;
-    for (int p = 0; p < K; p++) {
-        for (int q = 0; q < K; q++) blob[D.o_m + p * K + q] = mm[(size_t)p * K + q];
-        blob[D.o_A + p] = A[p];
-        blob[D.o_sm + p] = P.sm[p];
-        blob[D.o_cd0 + p] = P.cd[p];
-        blob[D.o_cdB + p] = P.cdBefore[p];
-        blob[D.o_cdA + p] = P.cdAfter[p];
-        blob[D.o_startN + p] = P.startLD[p] * (double)P.sizes[p];
-        blob[D.o_endN + p] = P.endLD[p] * (double)P.sizes[p];
-        blob[D.o_size + p] = (double)P.sizes[p];
-    }
     CK(cudaMemcpyAsync((void *)(h->st.params + (size_t)pp * D.blob), blob.data(), (size_t)D.blob * 8,
                        cudaMemcpyHostToDevice, h->stream));
     // live contact density: first upload sets every deme, later uploads only the masked ones
@@ -275,6 +284,91 @@ int vgsim_upload_params(vgsim_handle h, int pp, const double *b, const double *d
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
     P.uploaded = true;
+    return 0;
+}
+
+int vgsim_upload_param_grid(vgsim_handle h, int base_pp, int n_axes, const int32_t *axis_len, const int64_t *patch_off,
+                            const int64_t *patch_idx, const double *patch_val, int64_t first_point, int dst_pp0,
+                            int n_points) {
+    if (base_pp < 0 || base_pp >= h->n_pp) return fail("base parameter point out of range");
+    if (n_points < 1 || dst_pp0 < 0 || dst_pp0 > h->n_pp - n_points) return fail("destination parameter points out of range");
+    if (n_axes < 0) return fail("number of axes must be >= 0");
+    HostParams &B = host_params(h, base_pp);
+    if (!B.uploaded) return fail("base parameter point was not uploaded (vgsim_upload_params)");
+    const Dims &D = h->D;
+    auto g = std::make_shared<ParamGrid>();
+    long long total = 1, nv = 0;
+    for (int a = 0; a < n_axes; a++) {
+        if (axis_len[a] < 1) return fail("axis lengths must be >= 1");
+        if (total > (1LL << 62) / axis_len[a]) return fail("the grid has more than 2^62 points");
+        total *= axis_len[a];
+        nv += axis_len[a];
+    }
+    if (first_point < 0 || first_point > total - n_points) return fail("grid points out of range");
+    if (patch_off[0] != 0) return fail("patch offsets must start at 0");
+    for (long long j = 0; j < nv; j++)
+        if (patch_off[j + 1] < patch_off[j]) return fail("patch offsets must not decrease");
+    const long long nsrc = src_off(D, NSRC), ne = patch_off[nv];
+    for (long long k = 0; k < ne; k++)
+        if (patch_idx[k] < 0 || patch_idx[k] >= nsrc) return fail("patch index out of range");
+    g->base = flatten(D, B);
+    g->axis_len.assign(axis_len, axis_len + n_axes);
+    g->off.assign(patch_off, patch_off + nv + 1);
+    g->idx.assign(patch_idx, patch_idx + ne);
+    g->val.assign(patch_val, patch_val + ne);
+    CK(cudaSetDevice(h->device));
+    GridArgs a;
+    a.n_axes = n_axes;
+    a.first_point = first_point;
+    a.dst_pp0 = dst_pp0;
+    a.n_points = n_points;
+    a.nslots = param_grid_slots(h->num_sms, n_points);
+    Scratch<double> dbase, dval, dslots;
+    Scratch<int> dlen, derr, dflag;
+    Scratch<long long> doff, didx;
+    if (dbase.alloc(nsrc) || dlen.alloc(n_axes) || doff.alloc(nv + 1) || didx.alloc(ne) || dval.alloc(ne) ||
+        dslots.alloc((size_t)a.nslots * nsrc) || derr.alloc(n_points) || dflag.alloc(1))
+        return 1;
+    CK(cudaMemcpyAsync(dbase, g->base.data(), nsrc * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(dlen, axis_len, (size_t)n_axes * 4, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(doff, patch_off, (nv + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(didx, patch_idx, ne * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(dval, patch_val, ne * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemsetAsync(dflag, 0, 4, h->stream));
+    a.base = dbase, a.axis_len = dlen, a.off = doff, a.idx = didx, a.val = dval, a.slots = dslots, a.err = derr;
+    a.flag = dflag;
+    cudaError_t e = launch_param_grid(h->st, a, h->stream);
+    if (e != cudaSuccess) return fail(std::string("parameter grid kernels: ") + cudaGetErrorString(e));
+    h->launches += 3;
+    std::vector<int> err(n_points);
+    CK(cudaMemcpyAsync(err.data(), derr, (size_t)n_points * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int i = 0; i < n_points; i++) {
+        if (!err[i]) continue;
+        const int b = err[i];
+        return fail("parameter grid point " + std::to_string(first_point + i) + ": " +
+                    (b & GRID_ERR_SUSC ? "susceptibility type out of range"
+                     : b & GRID_ERR_SIZES ? "population sizes must be in [1, 2^31-1]"
+                     : b & GRID_ERR_MIG_SUM ? "the migration probabilities out of a population sum to more than 1"
+                                            : "a population's probability of staying (diagonal of the migration matrix) "
+                                              "must be more than 1e-15"));
+    }
+    for (int i = 0; i < n_points; i++) {
+        HostParams &P = h->hp[dst_pp0 + i];
+        P = HostParams();
+        P.uploaded = true;
+        P.grid = g;
+        P.grid_point = first_point + i;
+    }
+    return 0;
+}
+
+int vgsim_get_params(vgsim_handle h, int pp, double *blob_out) {
+    if (pp < 0 || pp >= h->n_pp) return fail("parameter point out of range");
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(blob_out, h->st.params + (size_t)pp * h->D.blob, (size_t)h->D.blob * 8, cudaMemcpyDeviceToHost,
+                       h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
@@ -890,7 +984,7 @@ int vgsim_get_multievents(vgsim_handle h, int r, int64_t n, int64_t *num, double
     std::vector<int32_t> cnt((size_t)n);
     std::vector<double> tt((size_t)L * 2);
     if (vgsim_get_tau_log(h, r, L, cnt.data(), tt.data())) return 1;
-    const HostParams &P = h->hp[h->rep_pp_host[r]];  // suscType of THIS replicate's parameter point (sweeps)
+    const HostParams &P = host_params(h, h->rep_pp_host[r]);  // suscType of THIS replicate's parameter point (sweeps)
     const int K = D.K, H = D.H, S = D.S, U = D.U;
     int64_t k = 0;
     auto put = [&](int64_t nn, double t, int ty, int a, int b, int c, int d2) {

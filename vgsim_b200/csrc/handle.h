@@ -1,16 +1,44 @@
 // Host-side handle behind the C ABI (include/vgsim_b200.h).
 #pragma once
 #include <cuda_runtime.h>
+#include <memory>
 #include <string>
 #include <vector>
 #include "common.cuh"
 
 namespace vg {
 
+// One vgsim_upload_param_grid call: the base point's source arrays (concatenated in vgsim_upload_params order, fp64) and
+// the patch tables, from which the host record of any of its points is rebuilt on demand.
+struct ParamGrid {
+    std::vector<double> base;
+    std::vector<int> axis_len;
+    std::vector<long long> off, idx;
+    std::vector<double> val;
+};
+
 struct HostParams {  // host copy of one parameter point in the reference's layouts
     std::vector<double> b, d, s, mRate, hapMutType, sigma, T, m, cd, cdBefore, cdAfter, startLD, endLD, sm;
     std::vector<long long> suscType, sizes;
     bool uploaded = false;
+    std::shared_ptr<const ParamGrid> grid;  // set: a grid point whose arrays above are not filled in yet
+    long long grid_point = 0;               // its global index in the grid
+};
+
+// Arguments of the parameter-grid kernels (param_grid_kernel.cu); device pointers.
+enum { GRID_ERR_SUSC = 1, GRID_ERR_SIZES = 2, GRID_ERR_MIG_SUM = 4, GRID_ERR_MIG_DIAG = 8 };
+struct GridArgs {
+    const double *base;  // [nsrc] the base point's source arrays, concatenated
+    int n_axes;
+    const int *axis_len;                  // [n_axes]
+    const long long *off, *idx;           // [sum axis_len + 1], [off[sum]]
+    const double *val;                    // [off[sum]]
+    long long first_point;
+    int dst_pp0, n_points;
+    double *slots;  // [nslots][nsrc] one assembled point per CTA
+    int nslots;
+    int *err;       // [n_points] GRID_ERR_* bits of each point
+    int *flag;      // [1] non-zero when any point failed
 };
 
 struct GenealogyBuffers {
@@ -115,5 +143,7 @@ cudaError_t launch_rates_tap(const DevState &st, int r, double *ev, double *hp, 
 cudaError_t launch_rates_large(const DevState &st, const DLLayout &L, double *slice, int r, double *ev, double *hp,
                                double *popRate, double *migPop, double *totals, cudaStream_t stream);
 bool tau_fits(const Dims &D, int uniform_pp);
+int param_grid_slots(int num_sms, int n_points);
+cudaError_t launch_param_grid(const DevState &st, const GridArgs &g, cudaStream_t stream);
 
 }  // namespace vg
