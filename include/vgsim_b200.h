@@ -263,8 +263,14 @@ int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step
  * Bits 2 and 3 pick the kernel mapping (scheduling only, same log bit for bit): by default a batch small enough to
  * be resident as 256-thread teams runs on the team kernel, larger batches on the warp-per-replicate kernel; bit 2
  * forces the former, bit 3 the latter.  Bits 4 and 5 switch off the warp kernel's lockstep generations and its
- * size-sorted replicate schedule (scheduling only as well; tests check that the log does not change). */
+ * size-sorted replicate schedule (scheduling only as well; tests check that the log does not change).  Bit 6 runs the
+ * warp kernel instance that reads the model dimensions at run time even where one with the shape compiled in exists
+ * (same log bit for bit; see vgsim_tau_fixed_shape). */
 int vgsim_set_tau_variant(vgsim_handle h, int variant);
+/* Which warp kernel instance the last tau launch of this handle ran: U << 16 | K << 8 | S of the model shape it was
+ * compiled for ((3, 10, 3) and (2, 10, 3) have one), 0 for an instance that reads the shape at run time (every
+ * other shape, variant bit 6, the team kernel). */
+int vgsim_tau_fixed_shape(vgsim_handle h);
 /* Parity tap of the direct method.  Bit 0: vgsim_simulate_direct and vgsim_rates use the large-state kernel (sum
  * trees in device memory) on every shape, not only on shapes whose rate hierarchy exceeds one SM's shared memory.
  * Default 0.  Tests compare the two kernels in distribution and the trees with the reference's rates. */

@@ -39,7 +39,7 @@ def _load():
         # in-tree build (nvcc cross-compiles sm_100a without a GPU); raises if nvcc is unavailable
         _build.build()
     lib = ctypes.CDLL(LIB_PATH)
-    if not hasattr(lib, "vgsim_upload_param_grid") and LIB_PATH == _build.LIB and _build.have_nvcc():
+    if not hasattr(lib, "vgsim_tau_fixed_shape") and LIB_PATH == _build.LIB and _build.have_nvcc():
         # a library built from older sources (it lacks the newest entry point): rebuild once and load the new file
         del lib
         _build.build(force=True)
@@ -93,6 +93,7 @@ def _load():
         "vgsim_launch_count": (c_int64, [P]),
         "vgsim_set_tau_variant": (c_int, [P, c_int]),
         "vgsim_set_direct_variant": (c_int, [P, c_int]),
+        "vgsim_tau_fixed_shape": (c_int, [P]),
         "vgsim_debug_tau_phases": (c_int, [P, P, c_int]),
         "vgsim_debug_tau_cta_end": (c_int, [P, P, c_int]),
         "vgsim_last_kernel_ms": (c_int, [P, ctypes.POINTER(c_float)]),
@@ -451,6 +452,12 @@ class Handle:
         """0 = small mutation / out-migration groups drawn as one Poisson total + multinomial split (product path),
         1 = every channel drawn separately like the reference (parity tap)."""
         _ck(lib.vgsim_set_tau_variant(self._h, int(variant)))
+
+    def tau_fixed_shape(self):
+        """(U, K, S) compiled into the warp kernel instance the last tau launch ran, None when it read the shape at
+        run time (variant bit 6 forces that instance)."""
+        v = int(lib.vgsim_tau_fixed_shape(self._h))
+        return (v >> 16, (v >> 8) & 0xff, v & 0xff) if v else None
 
     def set_direct_variant(self, variant):
         """0 = the shared-memory direct kernel wherever a replicate's rates fit one SM's shared memory, the large-state

@@ -651,7 +651,8 @@ static int tau_call(Handle *h, int64_t iterations, int64_t sample_size, float ep
         next_timer(h);
         CK(cudaEventRecord(h->ev_k0, h->stream));
     }
-    cudaError_t e = launch_tau(h->st, a, h->stream, h->num_sms, h->tau_variant, uniform_pp(h), h->tau_order);
+    cudaError_t e = launch_tau(h->st, a, h->stream, h->num_sms, h->tau_variant, uniform_pp(h), h->tau_order,
+                                &h->tau_fixed_shape);
     if (e != cudaSuccess) return fail(std::string("tau kernel: ") + cudaGetErrorString(e));
     if (timed) {
         CK(cudaEventRecord(h->ev_k1, h->stream));
@@ -1114,11 +1115,13 @@ int vgsim_debug_tau_cta_end(vgsim_handle h, uint64_t *out1024, int reset) {
 }
 
 int vgsim_set_tau_variant(vgsim_handle h, int variant) {
-    if (variant < 0 || variant > 63 || (variant & 12) == 12)
-        return fail("tau variant must be 0..63 (bit 0: per-channel draws, bit 1: phase timing, bit 2: force the team kernel, bit 3: force the warp kernel, bit 4: free-running warps, bit 5: unsorted schedule)");
+    if (variant < 0 || variant > 127 || (variant & 12) == 12)
+        return fail("tau variant must be 0..127 (bit 0: per-channel draws, bit 1: phase timing, bit 2: force the team kernel, bit 3: force the warp kernel, bit 4: free-running warps, bit 5: unsorted schedule, bit 6: runtime-shape warp kernel)");
     h->tau_variant = variant;
     return 0;
 }
+
+int vgsim_tau_fixed_shape(vgsim_handle h) { return h->tau_fixed_shape; }
 
 int vgsim_set_direct_variant(vgsim_handle h, int variant) {
     if (variant < 0 || variant > 1) return fail("direct variant must be 0 or 1 (bit 0: the large-state kernel on every shape)");

@@ -78,6 +78,7 @@ struct Handle {
     long long launches = 0;
     int tau_variant = 0;  // 0 = aggregated small groups (product), 1 = one Poisson draw per channel (parity tap)
     int direct_variant = 0;  // bit 0: the large-state direct kernel on every shape (parity tap)
+    int tau_fixed_shape = 0;  // U << 16 | K << 8 | S of the compiled-in shape the last tau launch ran, 0: runtime shape
     double *dl_slices = nullptr;  // warp slices of the large-state direct kernel (allocated at its first call)
     size_t dl_slices_n = 0;       // doubles held
     bool state_set = false;
@@ -118,7 +119,7 @@ DLLayout dl_layout(const Dims &D);
 
 // kernels' host launchers (defined in the .cu files)
 cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant, int uniform_pp,
-                       int *order_buf);
+                       int *order_buf, int *fixed_shape);
 cudaError_t tau_phase_cycles(unsigned long long *out16, int reset);
 cudaError_t tau_cta_end(unsigned long long *out1024, int reset);
 cudaError_t launch_propensities(const DevState &st, int r, double *out, double *dI, double *dS, double *tau,

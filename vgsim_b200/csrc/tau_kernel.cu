@@ -376,8 +376,8 @@ __device__ __forceinline__ void q_pass(const Dims &D, const TauShared &s) {
 }
 
 // Mg[p,s] = sum_{t != p} eff[t,p] Sx[t,s] (needs only Sx; runs beside q_pass).  Same loop order in the warp kernel.
-template <class SH>
-__device__ __forceinline__ void mig_pressure(int i, const Dims &D, const SH &s, const double *eff) {
+template <class DIMS, class SH>
+__device__ __forceinline__ void mig_pressure(int i, const DIMS &D, const SH &s, const double *eff) {
     const int K = D.K, S = D.S;
     const int p = i / S, sn = i - p * S;
     double acc = 0.0;
@@ -390,8 +390,8 @@ __device__ __forceinline__ void mig_pressure(int i, const Dims &D, const SH &s, 
 // Net drift of infectious cell i = (p,h): force of infection (own deme + migration from every deme holding h),
 // removal, and mutation inflow from the haplotypes one substitution away that are present in the deme
 // (Propensities :2351-2417 summed per compartment).  Every sum runs in ascending index order.
-template <class SH>
-__device__ __forceinline__ double drift_I_cell(int i, const Dims &D, const SH &s, const double *eff) {
+template <class DIMS, class SH>
+__device__ __forceinline__ double drift_I_cell(int i, const DIMS &D, const SH &s, const double *eff) {
     const int K = D.K, H = D.H, U = D.U;
         const int p = i >> D.hshift, h = i & (H - 1);
         const double Iv = s.I[i];
@@ -458,8 +458,8 @@ __device__ __forceinline__ double drift_I_cell(int i, const Dims &D, const SH &s
 }
 
 // Net drift of susceptible compartment i = (p, sn)
-template <class SH>
-__device__ __forceinline__ double drift_S_cell(int i, const Dims &D, const SH &s, const double *eff) {
+template <class DIMS, class SH>
+__device__ __forceinline__ double drift_S_cell(int i, const DIMS &D, const SH &s, const double *eff) {
     const int K = D.K, S = D.S;
         const int p = i / S, sn = i - p * S;
         double phi = s.c[p] * s.Bp[i];
@@ -706,7 +706,8 @@ struct DrawGeom {
     int LC;    // channels owned by a cell
 };
 
-__device__ __forceinline__ DrawGeom draw_geom(const Dims &D) {
+template <class DIMS>
+__device__ __forceinline__ DrawGeom draw_geom(const DIMS &D) {
     DrawGeom g;
     g.LC = D.E + (D.K - 1) * D.S;
     g.NB1 = 1 + ((D.S + 3) >> 2);
@@ -732,8 +733,8 @@ static_assert(TAU_THETA_MUT < 10.0 && TAU_THETA_MIG < 10.0, "aggregated totals a
 // I b[h] m[p,p] eff[t,p] Sx[t,s] sigma[s,h], with the sum over targets taken once per leap and (deme, group):
 // sum_s sigma[s,h] Mg[p,s] -- S multiply-adds per cell instead of (K-1) S (the targets' Q[t,h] = sum_s Sx[t,s] sigma[s,h]
 // were 7 % of a dense leap's instructions in the warp kernel, whose Q table no longer fits when most haplotypes are present)
-template <class SH>
-__device__ __forceinline__ double mig_total(int p, int h, double Ii, const Dims &D, const SH &s, const double *eff) {
+template <class DIMS, class SH>
+__device__ __forceinline__ double mig_total(int p, int h, double Ii, const DIMS &D, const SH &s, const double *eff) {
     (void)eff;
     double acc = 0.0;
 #pragma unroll 1
@@ -743,8 +744,8 @@ __device__ __forceinline__ double mig_total(int p, int h, double Ii, const Dims 
 
 // One event of an aggregated out-migration total of cell (p,h): its local channel, or -1 when every weight is zero.
 // Shared by both kernels (same arithmetic, same pick for the same uniform).
-template <class SH>
-__device__ __forceinline__ int split_migration(int p, int h, double u, const Dims &D, const SH &s, const double *eff) {
+template <class DIMS, class SH>
+__device__ __forceinline__ int split_migration(int p, int h, double u, const DIMS &D, const SH &s, const double *eff) {
     const int K = D.K, H = D.H, S = D.S;
     double tot = 0.0;
 #pragma unroll 1
@@ -1297,11 +1298,24 @@ bool tau_fits(const Dims &D, int uniform_pp) {
     return tau_warp_fits(D, warp_layout(D, uniform_pp >= 0, uniform_pp >= 0 ? uniform_pp : 0, 227 * 1024));
 }
 
+// Warp kernel instances with the model shape compiled in (DimsC), all on the mask path with eff in shared memory:
+// T3 (3, 10, 3), the benchmark's model, and (2, 10, 3), the Table 3 model of the configs[4] sweep.  nullptr when the
+// shape is another one.
+template <int U, int K, int S>
+static const void *tau_warp_fixed(const Dims &D, bool prof) {
+    if (!DimsC<U, K, S>::matches(D)) return nullptr;
+    return prof ? (const void *)tau_warp_kernel<DimsC<U, K, S>, true, true, true>
+                : (const void *)tau_warp_kernel<DimsC<U, K, S>, false, true, true>;
+}
+
 // Default: the warp-per-replicate kernel (tau_warp.cuh), one CTA per SM with as many warps as the shared memory
-// holds (<= 14).  The team kernel (256-thread teams, CTA-wide generations) stays available as a parity tap:
-// variant bit 2 (vgsim_set_tau_variant); bit 3 forces the warp kernel.
+// holds (<= 14), with the model shape compiled in where an instance exists for it (variant bit 6: the runtime-shape
+// instance on every shape).  The team kernel (256-thread teams, CTA-wide generations) stays available as a parity tap:
+// variant bit 2 (vgsim_set_tau_variant); bit 3 forces the warp kernel.  *fixed_shape gets U << 16 | K << 8 | S of the
+// compiled-in shape that ran, 0 for a runtime-shape kernel.
 cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream, int num_sms, int variant, int uniform_pp,
-                       int *order_buf) {
+                       int *order_buf, int *fixed_shape) {
+    *fixed_shape = 0;
     if ((long long)st.D.K * st.D.H + st.D.K >= (1 << 20)) return cudaErrorInvalidValue;  // owner id is packed in 20 bits
     const size_t stride = tau_team_stride(st.D);
     int teams = (int)((227 * 1024 - TAU_CTA_TAIL) / stride);
@@ -1320,9 +1334,15 @@ cudaError_t launch_tau(const DevState &st, const SimArgs &a, cudaStream_t stream
         if (tau_warp_fits(st.D, L)) {
             const WS ws = make_ws(L, st.D);
             const bool prof = (variant & 2) != 0, masks = L.use_masks != 0;
-            const void *kern = L.has_eff ? (masks ? (prof ? (const void *)tau_warp_kernel<true, true, true> : (const void *)tau_warp_kernel<false, true, true>)
-                                                  : (prof ? (const void *)tau_warp_kernel<true, true, false> : (const void *)tau_warp_kernel<false, true, false>))
-                                         : (prof ? (const void *)tau_warp_kernel<true, false, false> : (const void *)tau_warp_kernel<false, false, false>);
+            const void *kern = nullptr;
+            if (L.has_eff && masks && !(variant & 64)) {
+                if ((kern = tau_warp_fixed<3, 10, 3>(st.D, prof))) *fixed_shape = 3 << 16 | 10 << 8 | 3;
+                else if ((kern = tau_warp_fixed<2, 10, 3>(st.D, prof))) *fixed_shape = 2 << 16 | 10 << 8 | 3;
+            }
+            if (!kern)
+                kern = L.has_eff ? (masks ? (prof ? (const void *)tau_warp_kernel<Dims, true, true, true> : (const void *)tau_warp_kernel<Dims, false, true, true>)
+                                          : (prof ? (const void *)tau_warp_kernel<Dims, true, true, false> : (const void *)tau_warp_kernel<Dims, false, true, false>))
+                                 : (prof ? (const void *)tau_warp_kernel<Dims, true, false, false> : (const void *)tau_warp_kernel<Dims, false, false, false>);
             cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total_bytes);
             if (e != cudaSuccess) return e;
             int grid = (st.R + L.nwarps - 1) / L.nwarps;

@@ -17,6 +17,12 @@
 // same summation orders, same Philox addressing (owner, leap, retry|epoch, block), same samplers -- a leap
 // is a pure function of (state, seed), so the two kernels produce the same log.  The team kernel stays as a
 // parity tap (variant bit 2).
+//
+// The kernel and its helpers are templated on the dims type: `Dims` reads the model shape at run time, `DimsC<U, K, S>`
+// has it compiled in (T3 (3, 10, 3) and the configs[4] model (2, 10, 3); launch_tau picks the instance, variant bit 6
+// forces the runtime one).  Same source, same arithmetic, same log; the fixed-shape instance does without the runtime
+// divisions of the item decode and the per-cell sums, the shape-derived values held in registers across the leap loop,
+// and the branches the shape never takes.
 #pragma once
 
 namespace vg {
@@ -49,6 +55,32 @@ struct WarpLayout {
     // n / d = __umulhi(n, m) for the small divisors of the item decode (n < 2^20, d <= 4096: exact)
     unsigned mS, mS1, mNBT, mG2, mnbm, mnbg, mK;
 };
+// The model dimensions as compile-time constants (make_dims' formulas) for the kernel instances of the common shapes.
+// Every dimension the leap loop reads is shadowed by a constant of the same name, so the helpers, templated on the dims
+// type, read D.K, D.H, ... alike for both: with a DimsC the divisions by K, S and 3U become multiplies, the loop bounds
+// and group sizes constants, the branches the shape never takes drop out, and nothing of it holds a register.  The
+// members that only the cold paths read (P, the blob offsets) stay those of the Dims it is built from.
+template <int U_, int K_, int S_>
+struct DimsC : Dims {
+    static constexpr int U = U_, K = K_, S = S_, H = 1 << (2 * U_), hshift = 2 * U_;
+    static constexpr int E = 2 + 3 * U + S, SS1 = S * (S - 1), PD = SS1 + H * E, NA = K * (K - 1) * S * H;
+    static constexpr int Pp = (NA + K * PD + 7) & ~7;
+    __device__ DimsC(const Dims &d) : Dims(d) {}
+    static bool matches(const Dims &d) {
+        return d.U == U && d.K == K && d.S == S && d.H == H && d.hshift == hshift && d.E == E && d.SS1 == SS1 &&
+               d.PD == PD && d.NA == NA && d.Pp == Pp;
+    }
+};
+// how the kernel holds its dimensions: the runtime shape by reference into its parameter block, a DimsC by value
+template <class DIMS>
+struct DimsRef {
+    using type = const DIMS;
+};
+template <>
+struct DimsRef<Dims> {
+    using type = const Dims &;
+};
+
 inline unsigned div_magic(int d) { return d > 1 ? (unsigned)((0x100000000ull + (unsigned)d - 1) / (unsigned)d) : 0u; }
 __device__ __forceinline__ int fdiv(int n, unsigned magic, int d) { return d > 1 ? (int)__umulhi((unsigned)n, magic) : n; }
 
@@ -306,8 +338,8 @@ static __device__ __noinline__ int w_lockdown_slow(const DevState &st, int r, co
     }
     return flips;
 }
-template <class WSQ>
-__device__ __forceinline__ int w_lockdown(const DevState &st, int r, const Dims &D, const WSQ &s, const double *pp,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ int w_lockdown(const DevState &st, int r, const DIMS &D, const WSQ &s, const double *pp,
                                           double *eff_g, double now) {
     int pred = 0;
 #pragma unroll 1
@@ -316,12 +348,12 @@ __device__ __forceinline__ int w_lockdown(const DevState &st, int r, const Dims 
         if ((ti > s.startN[p] && s.lock[p] == 0) || (ti < s.endN[p] && s.lock[p] == 1)) pred = 1;
     }
     if (!__any_sync(0xffffffffu, pred)) return 0;
-    return w_lockdown_slow(st, r, D, s, pp, eff_g, now);
+    return w_lockdown_slow(st, r, st.D, s, pp, eff_g, now);  // out of line: the runtime Dims, not a local copy
 }
 
 // stage one parameter point (blob layout of common.cuh) into a shared-memory parameter block
-template <class WSQ>
-__device__ __forceinline__ void w_load_params(const Dims &D, const WSQ &s, const double *pp, int t, int n) {
+template <class DIMS, class WSQ>
+__device__ __forceinline__ void w_load_params(const DIMS &D, const WSQ &s, const double *pp, int t, int n) {
     const int K = D.K, H = D.H, S = D.S, U = D.U;
 #pragma unroll 1
     for (int i = t; i < H; i += n) {
@@ -374,8 +406,8 @@ __device__ __forceinline__ void w_load_params(const Dims &D, const WSQ &s, const
 // Ordered compaction of the infectious cells of the CURRENT counts (+ upd when APPLY): act[] ascending, dstart[],
 // presence masks / counts, per-deme totals, the ascending list of haplotypes present anywhere.  Returns the
 // number of infectious cells; nhap gets the number of present haplotypes.  One warp, ends with __syncwarp().
-template <class WSQ, bool APPLY>
-__device__ __forceinline__ int w_lists(const Dims &D, const WSQ &s, int &nhap, RowWiper &wp, int wk, int n32) {
+template <class DIMS, class WSQ, bool APPLY>
+__device__ __forceinline__ int w_lists(const DIMS &D, const WSQ &s, int &nhap, RowWiper &wp, int wk, int n32) {
     const int lane = threadIdx.x & 31, K = D.K, H = D.H, KH = K * H;
 #pragma unroll 1
     for (int i = lane; i < H; i += 32) s.colcnt[i] = 0;  // (= colmask on the mask path)
@@ -489,8 +521,8 @@ __device__ __forceinline__ double warp_min_d(double v) {
 }
 
 // Drifts and tau (ChooseTau :2432-2450) of the warp's state; same sums as the team kernel's drifts_and_tau.
-template <class WSQ>
-__device__ __forceinline__ double w_drifts_and_tau(const Dims &D, const WSQ &s, const double *eff, int nhap, int nAct,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ double w_drifts_and_tau(const DIMS &D, const WSQ &s, const double *eff, int nhap, int nAct,
                                                    RowWiper &wp, int wk, int n32) {
     const int K = D.K, H = D.H, S = D.S, KS = K * S;
     const int lane = threadIdx.x & 31;
@@ -642,7 +674,8 @@ struct DrawState {  // warp-uniform registers of one attempt at a leap
 };
 
 // Philox domain and word index of the draw (owner, l)
-__device__ __forceinline__ void tw_addr(int owner, int l, const Dims &D, const DrawGeom &g, int &dom, int &q) {
+template <class DIMS>
+__device__ __forceinline__ void tw_addr(int owner, int l, const DIMS &D, const DrawGeom &g, int &dom, int &q) {
     const int KH = D.K * D.H;
     if (owner >= KH) {  // SUSCCHANGE channel l of a deme
         dom = l >> 2;
@@ -668,8 +701,8 @@ __device__ __forceinline__ void tw_addr(int owner, int l, const Dims &D, const D
 }
 
 // where the n events of channel (owner, l) go (cell_channel / susc_channel without the propensity) + the row index
-template <class WSQ>
-__device__ __forceinline__ int tw_channel_ids(int owner, int l, const Dims &D, const WSQ &s, const WarpLayout &L, Channel &ch) {
+template <class DIMS, class WSQ>
+__device__ __forceinline__ int tw_channel_ids(int owner, int l, const DIMS &D, const WSQ &s, const WarpLayout &L, Channel &ch) {
     const int K = D.K, H = D.H, S = D.S, KH = K * H;
     ch.i_dec = ch.i_inc = ch.i_chk = ch.s_dec = ch.s_inc = -1;
     ch.prop = 0.0;
@@ -713,8 +746,8 @@ __device__ __forceinline__ int tw_channel_ids(int owner, int l, const Dims &D, c
 // One event of the multinomial split of an aggregated total (split_total_impl of the team kernel, one event):
 // event e of the total of cell `owner` (kind 2: mutation group, 3: out-migration group) picks its channel with the
 // e-th 53-bit uniform of the group's split domain.  Returns the local channel or -1.
-template <class WSQ>
-__device__ __forceinline__ int tw_split_event(int owner, int kind, int e, const Dims &D, const WSQ &s, const double *eff,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ int tw_split_event(int owner, int kind, int e, const DIMS &D, const WSQ &s, const double *eff,
                                               const DrawGeom &g, PhiloxCtx &ctx) {
     const int K = D.K, H = D.H, S = D.S, U = D.U;
     const int p = owner >> D.hshift, h = owner & (H - 1);
@@ -744,8 +777,8 @@ __device__ __forceinline__ int tw_split_event(int owner, int kind, int e, const 
 
 // One round (<= 32, taken from the end of the list) of parked aggregated totals: every lane splits one total, one event
 // per iteration.
-template <class WSQ>
-__device__ __forceinline__ void w_split_parked(int *row, const Dims &D, const WSQ &s, const double *eff, const DrawGeom &g,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ void w_split_parked(int *row, const DIMS &D, const WSQ &s, const double *eff, const DrawGeom &g,
                                                const WarpLayout &L, PhiloxCtx &ctx, LeapTally &tr, DrawState &q) {
     const int lane = threadIdx.x & 31;
     const int take = q.nsq < 32 ? q.nsq : 32;
@@ -776,8 +809,8 @@ __device__ __forceinline__ void w_split_parked(int *row, const Dims &D, const WS
 //     (they ran with 1.5 of 32 lanes when every drain split its own few totals, ncu profiles/r2_c_*);
 //   * PTRS entries in rounds of 32, one inlined copy of the sampler.
 #define TW_SQCAP 64
-template <class WSQ>
-__device__ __forceinline__ void w_drain(int *row, const Dims &D, const WSQ &s, const double *eff, const DrawGeom &g,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ void w_drain(int *row, const DIMS &D, const WSQ &s, const double *eff, const DrawGeom &g,
                                         const WarpLayout &L, PhiloxCtx &ctx, LeapTally &tr, DrawState &q, bool final) {
     const int lane = threadIdx.x & 31;
     const unsigned lt = (1u << lane) - 1u;
@@ -861,8 +894,8 @@ struct RoundOut {  // what a lane's block leaves for the queue
 // One round of 32 block items: lambdas, the Philox block, early-outs; returns the number of queue entries the round
 // needs (w_push stores them).  mode 0: the primary item space [cells: block 0 | cells x transmission blocks | demes x
 // SUSCCHANGE blocks]; mode 1: the blocks of the groups listed in the expansion queues [mutation | out-migration].
-template <class WSQ>
-__device__ __forceinline__ int w_round(int item, int mode, int nAct, double tau, int variant, const Dims &D, const WSQ &s,
+template <class DIMS, class WSQ>
+__device__ __forceinline__ int w_round(int item, int mode, int nAct, double tau, int variant, const DIMS &D, const WSQ &s,
                                        const double *eff, const DrawGeom &g, const WarpLayout &L, PhiloxCtx &ctx,
                                        DrawState &q, RoundOut &ro) {
     const int lane = threadIdx.x & 31;
@@ -1046,12 +1079,12 @@ __global__ void __launch_bounds__(1024) tau_order_kernel(int R, int KH, const in
     }
 }
 
-template <bool PROF, bool EFFS, bool MASKS>
+template <class DIMS, bool PROF, bool EFFS, bool MASKS>
 __global__ void __launch_bounds__(TW_MAX_WARPS * 32, 1)
     tau_warp_kernel(const __grid_constant__ DevState st, const __grid_constant__ SimArgs a,
                     const __grid_constant__ WarpLayout L, const __grid_constant__ WSX<MASKS> s, const int variant,
                     const int *__restrict__ order) {
-    const Dims &D = st.D;
+    typename DimsRef<DIMS>::type D = st.D;
     const int K = D.K, H = D.H, S = D.S, KH = K * H, KS = K * S;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
     const DrawGeom g = draw_geom(D);
@@ -1155,7 +1188,7 @@ __global__ void __launch_bounds__(TW_MAX_WARPS * 32, 1)
         RowWiper wp;
         wp.idle();
         int pre_row = -1;  // leap whose row the wiper is working on / has finished
-        int nAct = w_lists<WSX<MASKS>, false>(D, s, nhap, wp, 0, n32);
+        int nAct = w_lists<DIMS, WSX<MASKS>, false>(D, s, nhap, wp, 0, n32);
 
         bool restarted = false;
         if (lane < 6) s.tally64[lane] = 0;
@@ -1322,7 +1355,7 @@ __global__ void __launch_bounds__(TW_MAX_WARPS * 32, 1)
                     // ---- 5. apply (UpdateCompartmentCounts_tau, :2536-2593) fused with the list rebuild
 #pragma unroll 1
                     for (int i = lane; i < KS; i += 32) s.Sx[i] += (double)s.dSx[i];
-                    nAct = w_lists<WSX<MASKS>, true>(D, s, nhap, wp, 1, n32);
+                    nAct = w_lists<DIMS, WSX<MASKS>, true>(D, s, nhap, wp, 1, n32);
                     if (lane == 0) {
                         double *tau_tt = st.tau_tt + ((size_t)r * st.leap_cap + leaps) * 2;
                         tau_tt[0] = t;
@@ -1353,7 +1386,7 @@ __global__ void __launch_bounds__(TW_MAX_WARPS * 32, 1)
 #pragma unroll 1
                 for (int i = lane; i < KS; i += 32) s.Sx[i] = (double)st.initSx[(size_t)r * KS + i];
                 __syncwarp();
-                nAct = w_lists<WSX<MASKS>, false>(D, s, nhap, wp, 0, n32);
+                nAct = w_lists<DIMS, WSX<MASKS>, false>(D, s, nhap, wp, 0, n32);
                 flips_total += w_lockdown(st, r, D, s, pp, eff_g, t);
                 good_attempt = 0;
                 dbase = 0;  // the archive of the wiped leaps goes with them
