@@ -225,7 +225,8 @@ int64_t vgsim_num_migrations(vgsim_handle h, int replicate);
 int vgsim_get_migrations(vgsim_handle h, int replicate, int64_t *node, double *time, int64_t *old_pop,
                          int64_t *new_pop);
 
-/* Fixed-size per-replicate summary vector (device-resident; what the multi-GPU all-gather moves):
+/* Fixed-size per-replicate summary vector (device-resident; what the multi-GPU all-gather moves, together with the
+ * time-resolved rows of vgsim_trajectories_dev and vgsim_lineages_through_time_dev when a sweep wants them):
  * counters, final time, and tree statistics when a genealogy exists.  out[R][VGSIM_NSUMMARY] f64:
  *   [0..11] the VGSIM_NCOUNTERS counters, [12] current time, [13] tree nodes (2n-1), [14] tree height,
  *   [15] total branch length, [16] roots (1 = fully coalesced), [17] mutation rows, [18] migration rows,
@@ -253,6 +254,30 @@ int vgsim_summaries_dev(vgsim_handle h, void **dev_ptr);
 int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step_num, int64_t *infectious,
                           int64_t *susceptible, int64_t *removed, int64_t *sampled, double *time_points,
                           int32_t *last_point);
+
+/* Trajectories of every replicate on ONE time grid shared by all of them, one pass over each event log (the walk of
+ * vgsim_epidemic_curves: direct rows, dense MULTITYPE rows, archived leaps; replicates whose counts exceed one SM's shared
+ * memory replay in device scratch slices).  times[T]: absolute times, finite, strictly increasing, 1 <= T <= 2^30.  Row
+ * j of replicate r is the state after every log row with time <= times[j], starting from the state vgsim_epidemic_curves
+ * starts from, as 2K + 2H int64 in this order:
+ *   infectious per deme [K] (sum over haplotypes), infectious per haplotype [H] (sum over demes),
+ *   samplings per deme [K] and per haplotype [H], cumulative since the start of the log.
+ * A point with times[j] > currentTime[r] was not simulated for that replicate: every entry of its row is -1.
+ * out[R][T][2K + 2H].  vgsim_trajectories_dev returns the DEVICE pointer of the same rows instead (a buffer owned by the
+ * handle, grown when needed, valid until the next vgsim_trajectories* call or destroy); the rows are fixed-size per
+ * replicate, so a multi-GPU all-gather can move them like the summaries.  vgsim_last_kernel_ms reports the kernel. */
+int vgsim_trajectories(vgsim_handle h, const double *times, int64_t T, int64_t *out);
+int vgsim_trajectories_dev(vgsim_handle h, const double *times, int64_t T, void **dev_ptr);
+
+/* Lineages through time of every replicate's genealogy (after vgsim_genealogy; fails with a message before one, or after
+ * a later simulate call) on the grid times[T] (same rules as vgsim_trajectories, T <= 32768):
+ *   out[r][j] = #{ node i : time[i] >= times[j] and (parent[i] < 0 or time[parent[i]] < times[j]) }
+ * with absolute node times as vgsim_get_tree returns them; every root of a forest counts its lineage.  A replicate
+ * without a tree (summaries[13] == 0) gets a row of zeros.  out[R][T] int64; vgsim_lineages_through_time_dev returns the
+ * DEVICE pointer of the same rows (owned by the handle, valid until the next vgsim_lineages_through_time* call or
+ * destroy).  vgsim_last_kernel_ms reports the kernel. */
+int vgsim_lineages_through_time(vgsim_handle h, const double *times, int64_t T, int64_t *out);
+int vgsim_lineages_through_time_dev(vgsim_handle h, const double *times, int64_t T, void **dev_ptr);
 
 /* Parity tap.  Variant 0 (default, product): per infectious cell the kernel draws ONE Poisson for the total of
  * its mutation channels and ONE for the total of its out-migration channels whenever that total's lambda is
@@ -287,7 +312,7 @@ int vgsim_debug_tau_cta_end(vgsim_handle h, uint64_t *out1024, int reset);
 
 /* Launch accounting: kernels launched by this handle since creation. */
 int64_t vgsim_launch_count(vgsim_handle h);
-/* Device time of the LAST hot kernel (tau / direct / epidemic curves), bracketed by CUDA events on the handle's
+/* Device time of the LAST hot kernel (tau / direct / epidemic curves / trajectories / lineages through time), bracketed by CUDA events on the handle's
  * stream inside vgsim_simulate_* (replaces the reference's time.time() pair, src/_interface.py:821-827).
  * Blocks until that kernel has finished. */
 int vgsim_last_kernel_ms(vgsim_handle h, float *ms);

@@ -39,7 +39,7 @@ def _load():
         # in-tree build (nvcc cross-compiles sm_100a without a GPU); raises if nvcc is unavailable
         _build.build()
     lib = ctypes.CDLL(LIB_PATH)
-    if not hasattr(lib, "vgsim_tau_fixed_shape") and LIB_PATH == _build.LIB and _build.have_nvcc():
+    if not hasattr(lib, "vgsim_lineages_through_time_dev") and LIB_PATH == _build.LIB and _build.have_nvcc():
         # a library built from older sources (it lacks the newest entry point): rebuild once and load the new file
         del lib
         _build.build(force=True)
@@ -90,6 +90,10 @@ def _load():
         "vgsim_epidemic_curves": (c_int, [P, c_int, c_int, c_int, P, P, P, P, P, P]),
         "vgsim_summaries": (c_int, [P, P]),
         "vgsim_summaries_dev": (c_int, [P, ctypes.POINTER(c_void_p)]),
+        "vgsim_trajectories": (c_int, [P, P, c_int64, P]),
+        "vgsim_trajectories_dev": (c_int, [P, P, c_int64, ctypes.POINTER(c_void_p)]),
+        "vgsim_lineages_through_time": (c_int, [P, P, c_int64, P]),
+        "vgsim_lineages_through_time_dev": (c_int, [P, P, c_int64, ctypes.POINTER(c_void_p)]),
         "vgsim_launch_count": (c_int64, [P]),
         "vgsim_set_tau_variant": (c_int, [P, c_int]),
         "vgsim_set_direct_variant": (c_int, [P, c_int]),
@@ -136,6 +140,24 @@ def _p(a):
 
 def _arr(a, dtype):
     return None if a is None else np.ascontiguousarray(a, dtype=dtype)
+
+
+def time_grid(times):
+    """`times` as the contiguous float64 grid vgsim_trajectories / vgsim_lineages_through_time take: one dimension, at
+    least one point, finite and strictly increasing values (ValueError otherwise; the C ABI checks the same rules)."""
+    t = np.ascontiguousarray(times, dtype=np.float64)
+    if t.ndim != 1:
+        raise ValueError("time grid must be one-dimensional (got shape %s)" % (t.shape,))
+    if t.size == 0:
+        raise ValueError("time grid needs at least one point")
+    bad = np.flatnonzero(~np.isfinite(t))
+    if bad.size:
+        raise ValueError("time grid: point %d (%r) is not finite" % (bad[0], t[bad[0]]))
+    bad = np.flatnonzero(np.diff(t) <= 0)
+    if bad.size:
+        raise ValueError("time grid must be strictly increasing (point %d, %r, is not after point %d, %r)"
+                         % (bad[0] + 1, t[bad[0] + 1], bad[0], t[bad[0]]))
+    return t
 
 
 class Handle:
@@ -412,6 +434,41 @@ class Handle:
     def summaries_dev_ptr(self):
         p = c_void_p()
         _ck(lib.vgsim_summaries_dev(self._h, ctypes.byref(p)))
+        return p.value
+
+    def trajectories(self, times):
+        """Every replicate's epidemic on the shared grid `times` (include/vgsim_b200.h: vgsim_trajectories): dict of int64
+        arrays infectious_deme [R, T, K], infectious_hap [R, T, H], sampled_deme [R, T, K], sampled_hap [R, T, H] (state
+        after every log row with time <= times[j]; samplings cumulative since the log start).  Rows of points after a
+        replicate's current time are -1."""
+        t = time_grid(times)
+        K, H = self.K, self.H
+        out = np.empty((self.R, t.size, 2 * (K + H)), np.int64)
+        _ck(lib.vgsim_trajectories(self._h, _p(t), t.size, _p(out)))
+        return {"infectious_deme": out[..., :K].copy(), "infectious_hap": out[..., K:K + H].copy(),
+                "sampled_deme": out[..., K + H:2 * K + H].copy(), "sampled_hap": out[..., 2 * K + H:].copy()}
+
+    def trajectories_dev_ptr(self, times):
+        """Device pointer of the rows of `trajectories(times)`, int64 [R, T, 2K + 2H] in the order infectious per deme,
+        per haplotype, sampled per deme, per haplotype (owned by the handle, valid until the next call)."""
+        t = time_grid(times)
+        p = c_void_p()
+        _ck(lib.vgsim_trajectories_dev(self._h, _p(t), t.size, ctypes.byref(p)))
+        return p.value
+
+    def lineages_through_time(self, times):
+        """Lineages of every replicate's genealogy alive at each grid time, int64 [R, T] (zeros for a replicate without
+        a tree; include/vgsim_b200.h: vgsim_lineages_through_time)."""
+        t = time_grid(times)
+        out = np.empty((self.R, t.size), np.int64)
+        _ck(lib.vgsim_lineages_through_time(self._h, _p(t), t.size, _p(out)))
+        return out
+
+    def lineages_through_time_dev_ptr(self, times):
+        """Device pointer of the rows of `lineages_through_time(times)`, int64 [R, T] (owned by the handle)."""
+        t = time_grid(times)
+        p = c_void_p()
+        _ck(lib.vgsim_lineages_through_time_dev(self._h, _p(t), t.size, ctypes.byref(p)))
         return p.value
 
     def last_kernel_ms(self):

@@ -685,6 +685,24 @@ class BirthDeathModel:
         include/vgsim_b200.h: vgsim_epidemic_curves)."""
         return self._handle.epidemic_curves(step_num, rep_first, rep_count, want)
 
+    def trajectories(self, times):
+        """Every replicate's epidemic on one time grid shared by all replicates, from one device pass over each log.
+
+        `times`: absolute times, finite and strictly increasing.  Returns a dict of int64 arrays ``infectious_deme``
+        [R, T, K], ``infectious_hap`` [R, T, H], ``sampled_deme`` [R, T, K] and ``sampled_hap`` [R, T, H]: the state after
+        every log row with time <= times[j], samplings counted from the start of the log.  A point after a replicate's
+        current time was not simulated for it: every entry of that replicate's row at that point is -1."""
+        if self._handle is None:
+            raise RuntimeError('Nothing was simulated. Use simulate() before trajectories().')
+        return self._handle.trajectories(times)
+
+    def lineages_through_time(self, times):
+        """int64 [R, T]: the lineages of each replicate's genealogy alive at times[j] (nodes with time >= times[j] whose
+        parent is older than times[j], or that are roots), times absolute like get_tree's; zeros for a replicate
+        without a tree.  Needs genealogy() after the last simulate()."""
+        self._require_tree()
+        return self._handle.lineages_through_time(times)
+
     def _lockdown_rows(self, pop, replicate):
         state, lp, lt = self._handle.get_lockdowns(replicate)
         return [[int(state[i]), float(lt[i])] for i in range(len(state)) if int(lp[i]) == pop]

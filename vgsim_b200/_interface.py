@@ -293,6 +293,18 @@ class Simulator:
         """Every compartment of a range of replicates on the reference's time grid, one device pass over the logs."""
         return self.simulation.epidemic_curves(step_num, rep_first, rep_count)
 
+    def trajectories(self, times):
+        """Infectious and cumulative sampled counts per deme and per haplotype of every replicate at the absolute times
+        `times` (finite, strictly increasing), one grid for all replicates: dict of int64 arrays infectious_deme
+        [R, T, K], infectious_hap [R, T, H], sampled_deme [R, T, K], sampled_hap [R, T, H].  A point after a replicate's
+        current time was not simulated for it, and every entry of its row there is -1."""
+        return self.simulation.trajectories(times)
+
+    def lineages_through_time(self, times):
+        """Lineages of each replicate's genealogy alive at the absolute times `times`, int64 [R, T] (after genealogy();
+        zeros for a replicate without a tree)."""
+        return self.simulation.lineages_through_time(times)
+
     def get_tree(self, replicate=0):
         return self.simulation.get_tree(replicate)
 

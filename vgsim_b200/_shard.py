@@ -32,9 +32,11 @@ def sweep_point(replicate_id, n_inner):
 
 
 def gather_summaries(local, world, group=None):
-    """All-gather per-replicate summary rows: `local` is a [n_local, NSUMMARY] torch tensor (CUDA for nccl,
-    CPU for gloo).  Returns [sum n_local, NSUMMARY] in global replicate order.  Ranks may own different
-    numbers of replicates (remainder ranks), so rows are padded to the maximum and trimmed after the gather."""
+    """All-gather per-replicate rows: `local` is a [n_local, ...] torch tensor of any trailing shape and dtype (CUDA for
+    nccl, CPU for gloo), e.g. the summaries [n_local, NSUMMARY] float64, trajectories [n_local, T, 2K + 2H] int64 or
+    lineages through time [n_local, T] int64.  Returns [sum n_local, ...] in global replicate order.  Ranks may own
+    different numbers of replicates (remainder ranks), so rows are padded to the maximum and trimmed after the
+    gather."""
     import torch
     import torch.distributed as dist
     if world == 1:

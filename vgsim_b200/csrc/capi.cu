@@ -1051,6 +1051,109 @@ int vgsim_get_lockdowns(vgsim_handle h, int r, int64_t *state, int64_t *pop, dou
     return 0;
 }
 
+}  // extern "C"
+
+// Replicates whose replay state does not fit one SM's shared memory replay in device slices: one per resident warp (at
+// most 16 per SM), at most half of the free device memory.  Nothing is allocated for a state that fits.
+static int replay_slices(Handle *h, size_t slice_bytes, int rep_count, const char *what, Scratch<unsigned char> &slices,
+                         int &nslices) {
+    nslices = 0;
+    if (slice_bytes <= 227 * 1024) return 0;
+    size_t fr = 0, tot = 0;
+    CK(cudaMemGetInfo(&fr, &tot));
+    const size_t nw = std::min<size_t>(std::min<size_t>(rep_count, (size_t)h->num_sms * 16), fr / 2 / slice_bytes);
+    if (nw < 1) return fail(std::string(what) + ": one replicate's counts exceed half of the free device memory");
+    if (slices.alloc(nw * slice_bytes)) return 1;
+    nslices = (int)nw;
+    return 0;
+}
+
+// A handle-owned device buffer of at least n elements (contents not kept when it grows).
+template <class T>
+static int ensure_buf(Handle *h, T **buf, size_t &cap, size_t n) {
+    if (n <= cap) return 0;
+    dfree(h, *buf);
+    *buf = nullptr;
+    cap = 0;
+    if (dalloc(h, buf, n)) return 1;
+    cap = n;
+    return 0;
+}
+
+// The caller's time grid: T >= 1 finite, strictly increasing values, at most max_points of them; copied to the handle's
+// grid buffer.
+static int upload_grid(Handle *h, const char *what, const double *times, int64_t T, int64_t max_points) {
+    const std::string w(what);
+    if (T < 1 || !times) return fail(w + ": the time grid needs at least one point");
+    if (T > max_points) return fail(w + ": at most " + std::to_string(max_points) + " grid points (got " + std::to_string(T) + ")");
+    for (int64_t j = 0; j < T; j++) {
+        if (!std::isfinite(times[j])) return fail(w + ": grid time " + std::to_string(j) + " is not finite");
+        if (j > 0 && !(times[j] > times[j - 1]))
+            return fail(w + ": grid times must be strictly increasing (point " + std::to_string(j) + " is not after point " +
+                        std::to_string(j - 1) + ")");
+    }
+    if (ensure_buf(h, &h->grid_buf, h->grid_cap, (size_t)T)) return 1;
+    CK(cudaMemcpyAsync(h->grid_buf, times, (size_t)T * 8, cudaMemcpyHostToDevice, h->stream));
+    return 0;
+}
+
+extern "C" {
+
+int vgsim_trajectories_dev(vgsim_handle h, const double *times, int64_t T, void **dev_ptr) {
+    CK(cudaSetDevice(h->device));
+    // grid indices are int on the device, and so is the point count of the launch
+    if (upload_grid(h, "trajectories", times, T, 1LL << 30)) return 1;
+    const Dims &D = h->D;
+    const size_t W = 2 * ((size_t)D.K + D.H);
+    if (ensure_buf(h, &h->traj_buf, h->traj_cap, (size_t)h->R * T * W)) return 1;
+    Scratch<unsigned char> d_slices;
+    int nslices = 0;
+    if (replay_slices(h, trajectories_slice_bytes(D), h->R, "trajectories", d_slices, nslices)) return 1;
+    next_timer(h);
+    CK(cudaEventRecord(h->ev_k0, h->stream));  // vgsim_last_kernel_ms then reports this kernel
+    cudaError_t e = launch_trajectories(h->st, h->grid_buf, (int)T, h->traj_buf, h->stream, h->num_sms, d_slices, nslices);
+    CK(cudaEventRecord(h->ev_k1, h->stream));
+    h->ev_valid = true;
+    h->launches++;
+    if (e != cudaSuccess) return fail(std::string("trajectories: ") + cudaGetErrorString(e));
+    if (nslices) CK(cudaStreamSynchronize(h->stream));  // the slices are freed on return
+    if (dev_ptr) *dev_ptr = h->traj_buf;
+    return 0;
+}
+
+int vgsim_trajectories(vgsim_handle h, const double *times, int64_t T, int64_t *out) {
+    if (vgsim_trajectories_dev(h, times, T, nullptr)) return 1;
+    const size_t W = 2 * ((size_t)h->D.K + h->D.H);
+    CK(cudaMemcpyAsync(out, h->traj_buf, (size_t)h->R * T * W * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int vgsim_lineages_through_time_dev(vgsim_handle h, const double *times, int64_t T, void **dev_ptr) {
+    CK(cudaSetDevice(h->device));
+    const GenealogyBuffers &G = h->gen;
+    if (!G.valid) return fail("lineages through time: no genealogy (call vgsim_genealogy after the last simulation)");
+    if (upload_grid(h, "lineages through time", times, T, ltt_max_points())) return 1;
+    if (ensure_buf(h, &h->ltt_buf, h->ltt_cap, (size_t)h->R * T)) return 1;
+    next_timer(h);
+    CK(cudaEventRecord(h->ev_k0, h->stream));
+    cudaError_t e = launch_ltt(h->st, G.node_off, G.parent, G.time, G.n_nodes, G.scratch, h->grid_buf, (int)T, h->ltt_buf,
+                               h->stream, h->num_sms);
+    CK(cudaEventRecord(h->ev_k1, h->stream));
+    h->ev_valid = true;
+    h->launches++;
+    if (e != cudaSuccess) return fail(std::string("lineages through time: ") + cudaGetErrorString(e));
+    if (dev_ptr) *dev_ptr = h->ltt_buf;
+    return 0;
+}
+
+int vgsim_lineages_through_time(vgsim_handle h, const double *times, int64_t T, int64_t *out) {
+    if (vgsim_lineages_through_time_dev(h, times, T, nullptr)) return 1;
+    CK(cudaMemcpyAsync(out, h->ltt_buf, (size_t)h->R * T * 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
 int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step_num, int64_t *infectious,
                           int64_t *susceptible, int64_t *removed, int64_t *sampled, double *time_points,
                           int32_t *last_point) {
@@ -1066,20 +1169,9 @@ int vgsim_epidemic_curves(vgsim_handle h, int rep_first, int rep_count, int step
     if ((infectious && d_inf.alloc(np * KH)) || (susceptible && d_sus.alloc(np * KS)) || (removed && d_rem.alloc(np * KH)) ||
         (sampled && d_smp.alloc(np * KH)) || (time_points && d_tp.alloc(np)) || (last_point && d_lp.alloc(rep_count)))
         return 1;
-    // replicates whose counts do not fit one SM's shared memory replay in device slices: one per resident warp (at most
-    // 16 per SM), at most half of the free device memory
-    const bool tallies = removed || sampled;
     Scratch<unsigned char> d_slices;
     int nslices = 0;
-    if (!curves_fit_shared(D, tallies)) {
-        size_t fr = 0, tot = 0;
-        CK(cudaMemGetInfo(&fr, &tot));
-        const size_t sb = curves_slice_bytes(D, tallies);
-        const size_t nw = std::min<size_t>(std::min<size_t>(rep_count, (size_t)h->num_sms * 16), fr / 2 / sb);
-        if (nw < 1) return fail("epidemic curves: one replicate's counts exceed half of the free device memory");
-        if (d_slices.alloc(nw * sb)) return 1;
-        nslices = (int)nw;
-    }
+    if (replay_slices(h, curves_slice_bytes(D, removed || sampled), rep_count, "epidemic curves", d_slices, nslices)) return 1;
     next_timer(h);
     CK(cudaEventRecord(h->ev_k0, h->stream));  // vgsim_last_kernel_ms then reports this kernel
     cudaError_t e = launch_curves(h->st, rep_first, rep_count, step_num, d_inf, d_sus, d_rem, d_smp, d_tp, d_lp, h->stream,

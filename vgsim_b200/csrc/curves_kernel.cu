@@ -21,6 +21,12 @@
 //
 // Roofline: HBM read of the log (B_leap = 4P + 16 bytes per leap, 16 B per direct event) + the snapshot writes
 // 8 * (3 K H + K S) * (step_num + 1) bytes per replicate.
+//
+// Trajectories (trajectories_kernel, TRAJ): the same walk on a grid the caller gives in absolute time, shared by every
+// replicate, with a snapshot of marginals instead of every cell: infectious per deme and per haplotype, cumulative
+// samplings per deme and per haplotype (2K + 2H int64 per point).  The slice holds I[K*H] and the K + H sampling
+// counters (no susceptible counts, no per-cell tallies); a point after the replicate's currentTime was not simulated
+// and is written as -1.  Roofline: the log once + 8 * (2K + 2H) * T bytes per replicate.
 #include "common.cuh"
 #include "handle.h"
 #include "logrec.cuh"
@@ -38,12 +44,36 @@ struct CurveArgs {
     int *last_point;                           // [rep_count] or null
 };
 
+struct TrajArgs {
+    const double *times;  // [step_num + 1] the grid, absolute times, strictly increasing
+    long long *out;       // [rep_count][step_num + 1][2K + 2H]
+};
+
+// TRAJ: no susceptible counts (Sx is not touched); rem = samplings per deme [K], smp = samplings per haplotype [H].
+template <bool TRAJ>
 __device__ __forceinline__ void curve_apply(int type, int hap, int pop, int nhap, int npop, long long n, int H, int S,
                                             unsigned long long *I, unsigned long long *Sx, unsigned long long *rem,
                                             unsigned long long *smp) {
     // unsigned wrap-around arithmetic == two's complement adds; the arrays are read back as signed
     const unsigned long long u = (unsigned long long)n, m = (unsigned long long)(-n);
     const int cell = pop * H + hap;
+    if constexpr (TRAJ) {
+        if (type == EV_BIRTH) {
+            atomicAdd(&I[cell], u);
+        } else if (type == EV_DEATH || type == EV_SAMPLING) {
+            atomicAdd(&I[cell], m);
+            if (type == EV_SAMPLING) {
+                atomicAdd(&rem[pop], u);
+                atomicAdd(&smp[hap], u);
+            }
+        } else if (type == EV_MUTATION) {
+            atomicAdd(&I[cell], m);
+            atomicAdd(&I[pop * H + nhap], u);
+        } else if (type == EV_MIGRATION) {
+            atomicAdd(&I[npop * H + hap], u);
+        }
+        return;
+    }
     if (type == EV_BIRTH) {  // hap infects a susceptible of group nhap in deme pop
         atomicAdd(&I[cell], u);
         atomicAdd(&Sx[pop * S + nhap], m);
@@ -66,20 +96,64 @@ __device__ __forceinline__ void curve_apply(int type, int hap, int pop, int nhap
     }
 }
 
+// One trajectory point from the warp's slice: o[2K + 2H] = infectious per deme, per haplotype, samplings per deme, per
+// haplotype (smp_deme and smp_hap are contiguous in the slice); every entry -1 for a point that was not simulated.
+// Called by the whole warp.
+__device__ __forceinline__ void traj_snapshot(const unsigned long long *I, const unsigned long long *smp, int K, int H,
+                                              bool after_end, long long *o) {
+    const int lane = threadIdx.x & 31;
+    if (after_end) {
+        for (int i = lane; i < 2 * (K + H); i += 32) o[i] = -1;
+        return;
+    }
+    if (H >= 32) {  // a warp reduction per deme
+        for (int p = 0; p < K; p++) {
+            unsigned long long s = 0ull;
+            for (int h = lane; h < H; h += 32) s += I[(size_t)p * H + h];
+#pragma unroll
+            for (int w = 16; w > 0; w >>= 1) s += __shfl_xor_sync(0xffffffffu, s, w);
+            if (lane == 0) o[p] = (long long)s;
+        }
+    } else {  // a lane per deme
+        for (int p = lane; p < K; p += 32) {
+            unsigned long long s = 0ull;
+            for (int h = 0; h < H; h++) s += I[p * H + h];
+            o[p] = (long long)s;
+        }
+    }
+    for (int h = lane; h < H; h += 32) {
+        unsigned long long s = 0ull;
+        for (int p = 0; p < K; p++) s += I[(size_t)p * H + h];
+        o[K + h] = (long long)s;
+    }
+    for (int i = lane; i < K + H; i += 32) o[K + H + i] = (long long)smp[i];
+}
+
 // The replay; GSLICE: the warps' slices live in gslices (one per warp of the grid, curves_large_kernel: replicates whose
-// counts do not fit one SM's shared memory), else in shared memory (curves_kernel).
-template <bool GSLICE>
-__device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs &a, int slice_bytes, unsigned char *gslices) {
+// counts do not fit one SM's shared memory), else in shared memory (curves_kernel).  TRAJ: the caller's grid ta.times
+// and marginal snapshots into ta.out (trajectories_kernel); a.step_num is then the grid's last index.
+template <bool GSLICE, bool TRAJ>
+__device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs &a, const TrajArgs &ta, int slice_bytes,
+                                            unsigned char *gslices) {
     const Dims &D = st.D;
     const int K = D.K, H = D.H, S = D.S, KH = K * H, KS = K * S;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
     unsigned long long *I = reinterpret_cast<unsigned long long *>(
         GSLICE ? gslices + (size_t)(blockIdx.x * nw + wid) * slice_bytes : curves_smem + (size_t)wid * slice_bytes);
-    const bool tallies = a.removed != nullptr || a.sampled != nullptr;
+    const bool tallies = !TRAJ && (a.removed != nullptr || a.sampled != nullptr);
     unsigned long long *Sx = I + KH, *rem = tallies ? Sx + KS : nullptr, *smp = tallies ? rem + KH : nullptr;
     // (channel, count) of the non-zero counts of the row being scanned
     int2 *queue = reinterpret_cast<int2 *>(tallies ? smp + KH : Sx + KS);
+    if constexpr (TRAJ) {  // I[KH], samplings per deme [K] and per haplotype [H], queue
+        Sx = nullptr;
+        rem = I + KH;
+        smp = rem + K;
+        queue = reinterpret_cast<int2 *>(smp + H);
+    }
     const int T = a.step_num;
+    // the walk may snapshot every point of the caller's grid; the reference's last point (= currentTime) is never
+    // crossed by a row and is written after the walk
+    const int walk_end = TRAJ ? T + 1 : T;
     for (int q = blockIdx.x * nw + wid; q < a.rep_count; q += gridDim.x * nw) {
         const int r = a.rep_first + q;
         const double *pp = st.params + (size_t)st.rep_pp[r] * D.blob;
@@ -92,7 +166,10 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
                 smp[i] = 0ull;
             }
         }
-        for (int i = lane; i < KS; i += 32) Sx[i] = (unsigned long long)S0[i];
+        if constexpr (TRAJ)
+            for (int i = lane; i < K + H; i += 32) rem[i] = 0ull;
+        else
+            for (int i = lane; i < KS; i += 32) Sx[i] = (unsigned long long)S0[i];
         __syncwarp();
         const long long n = st.counters[(size_t)r * NCOUNT + C_EVPTR];
         const double ct = st.time[r];
@@ -101,8 +178,18 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
         if (a.time_points)
             for (int j = lane; j <= T; j += 32) a.time_points[(size_t)q * (T + 1) + j] = ((double)j * ct) / (double)T;
         int point = 0;
+        auto grid = [&](int j) -> double {
+            if constexpr (TRAJ)
+                return ta.times[j];
+            else
+                return ((double)j * ct) / (double)T;
+        };
         auto snapshot = [&](int j) {  // coalesced copy of the current state into point j
             __syncwarp();
+            if constexpr (TRAJ) {
+                traj_snapshot(I, rem, K, H, ta.times[j] > ct, ta.out + ((size_t)q * (T + 1) + j) * (2 * (K + H)));
+                return;
+            }
             const size_t o = (size_t)q * (T + 1) + j;
             if (a.inf)
                 for (int i = lane; i < KH; i += 32) a.inf[o * KH + i] = (long long)I[i];
@@ -115,12 +202,14 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
         };
         // point advances while time_points[point] < t (reference :1975-1978); the state before the row is point's value
         auto advance = [&](double t) {
-            while (point != T && ((double)point * ct) / (double)T < t) {
+            while (point != walk_end && grid(point) < t) {
                 snapshot(point);
                 point++;
             }
         };
         for (long long base = 0; base < n; base += 32) {
+            if constexpr (TRAJ)
+                if (point == walk_end) break;  // every grid point is written: the rest of the log is not needed
             const long long i = base + lane;
             double t = 0.0;
             unsigned long long d = 0ull;
@@ -131,13 +220,13 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
             const int cnt = (int)((n - base < 32) ? n - base : 32);
             // does any row of this batch cross a grid point or carry a leap?  (times are non-decreasing)
             const double t_last = __shfl_sync(0xffffffffu, t, cnt - 1);
-            const bool crosses = point != T && ((double)point * ct) / (double)T < t_last;
+            const bool crosses = point != walk_end && grid(point) < t_last;
             const unsigned multi = __ballot_sync(0xffffffffu, i < n && (int)(d & 7) == EV_MULTITYPE);
             if (!crosses && multi == 0u) {  // fast path: 32 direct rows inside one grid interval, applied in parallel
                 if (i < n) {
                     int ty, hp_, pp_, nh, np_;
                     unpack_event(d, ty, hp_, pp_, nh, np_);
-                    curve_apply(ty, hp_, pp_, nh, np_, 1, H, S, I, Sx, rem, smp);
+                    curve_apply<TRAJ>(ty, hp_, pp_, nh, np_, 1, H, S, I, Sx, rem, smp);
                 }
                 continue;
             }
@@ -150,7 +239,7 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
                     if (lane == 0) {
                         int t2, hp_, pp_, nh, np_;
                         unpack_event(dk, t2, hp_, pp_, nh, np_);
-                        curve_apply(t2, hp_, pp_, nh, np_, 1, H, S, I, Sx, rem, smp);
+                        curve_apply<TRAJ>(t2, hp_, pp_, nh, np_, 1, H, S, I, Sx, rem, smp);
                     }
                     continue;
                 }
@@ -172,7 +261,7 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
                             if (en[u].x < 0) continue;
                             int mty, mh, mp, mnh, mnp;
                             decode_record(en[u].x, D, pp, mty, mh, mp, mnh, mnp);
-                            curve_apply(mty, mh, mp, mnh, mnp, (long long)en[u].y, H, S, I, Sx, rem, smp);
+                            curve_apply<TRAJ>(mty, mh, mp, mnh, mnp, (long long)en[u].y, H, S, I, Sx, rem, smp);
                         }
                     }
                     __syncwarp();
@@ -187,7 +276,7 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
                         const int2 en = queue[e];
                         int mty, mh, mp, mnh, mnp;
                         decode_record(en.x, D, pp, mty, mh, mp, mnh, mnp);
-                        curve_apply(mty, mh, mp, mnh, mnp, (long long)en.y, H, S, I, Sx, rem, smp);
+                        curve_apply<TRAJ>(mty, mh, mp, mnh, mnp, (long long)en.y, H, S, I, Sx, rem, smp);
                     }
                     __syncwarp();
                     qn = 0;
@@ -237,12 +326,22 @@ __device__ __forceinline__ void curves_body(const DevState &st, const CurveArgs 
 }
 
 __global__ void __launch_bounds__(512, 1) curves_kernel(const DevState st, const CurveArgs a, int slice_bytes) {
-    curves_body<false>(st, a, slice_bytes, nullptr);
+    curves_body<false, false>(st, a, TrajArgs{}, slice_bytes, nullptr);
 }
 
 __global__ void __launch_bounds__(512, 1) curves_large_kernel(const DevState st, const CurveArgs a, int slice_bytes,
                                                                unsigned char *gslices) {
-    curves_body<true>(st, a, slice_bytes, gslices);
+    curves_body<true, false>(st, a, TrajArgs{}, slice_bytes, gslices);
+}
+
+__global__ void __launch_bounds__(512, 1) trajectories_kernel(const DevState st, const CurveArgs a, const TrajArgs t,
+                                                               int slice_bytes) {
+    curves_body<false, true>(st, a, t, slice_bytes, nullptr);
+}
+
+__global__ void __launch_bounds__(512, 1) trajectories_large_kernel(const DevState st, const CurveArgs a, const TrajArgs t,
+                                                                     int slice_bytes, unsigned char *gslices) {
+    curves_body<true, true>(st, a, t, slice_bytes, gslices);
 }
 
 size_t curves_slice_bytes(const Dims &D, bool tallies) {
@@ -250,7 +349,39 @@ size_t curves_slice_bytes(const Dims &D, bool tallies) {
     return ((ncell * D.K * D.H + (size_t)D.K * D.S) * 8 + CURVE_QCAP * 8 + 15) & ~(size_t)15;
 }
 
-bool curves_fit_shared(const Dims &D, bool tallies) { return curves_slice_bytes(D, tallies) <= 227 * 1024; }
+size_t trajectories_slice_bytes(const Dims &D) {
+    return (((size_t)D.K * D.H + D.K + D.H) * 8 + CURVE_QCAP * 8 + 15) & ~(size_t)15;
+}
+
+// One launch of the replay: shared-memory slices when one replicate's fits one SM, else the gslices scratch.
+template <class Small, class Large, class... Extra>
+static cudaError_t launch_replay(Small small, Large large, size_t slice_bytes, int rep_count, cudaStream_t stream,
+                                 int num_sms, unsigned char *gslices, int nslices, const DevState &st, const CurveArgs &a,
+                                 Extra... extra) {
+    if (slice_bytes > 227 * 1024) {  // the state of one replicate does not fit one SM's shared memory
+        if (!gslices || nslices < 1) return cudaErrorInvalidValue;
+        int nw = (nslices + num_sms - 1) / num_sms;  // spread over the SMs, at most 16 warps per CTA
+        if (nw > 16) nw = 16;
+        int grid = nslices / nw;
+        if (grid > (rep_count + nw - 1) / nw) grid = (rep_count + nw - 1) / nw;
+        large<<<grid, nw * 32, 0, stream>>>(st, a, extra..., (int)slice_bytes, gslices);
+        return cudaGetLastError();
+    }
+    const int slice = (int)slice_bytes;
+    int nw = (227 * 1024) / slice;
+    if (nw > 16) nw = 16;
+    cudaError_t e = cudaFuncSetAttribute(small, cudaFuncAttributeMaxDynamicSharedMemorySize, nw * slice);
+    if (e != cudaSuccess) return e;
+    int per_sm = 1;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, small, nw * 32, (size_t)nw * slice);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    int grid = (rep_count + nw - 1) / nw;
+    if (grid > num_sms * per_sm) grid = num_sms * per_sm;
+    if (grid < 1) grid = 1;
+    small<<<grid, nw * 32, (size_t)nw * slice, stream>>>(st, a, extra..., slice);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_curves(const DevState &st, int rep_first, int rep_count, int step_num, long long *inf, long long *sus,
                           long long *removed, long long *sampled, double *time_points, int *last_point,
@@ -259,30 +390,18 @@ cudaError_t launch_curves(const DevState &st, int rep_first, int rep_count, int 
     a.rep_first = rep_first; a.rep_count = rep_count; a.step_num = step_num;
     a.inf = inf; a.sus = sus; a.removed = removed; a.sampled = sampled;
     a.time_points = time_points; a.last_point = last_point;
-    const bool tallies = removed || sampled;
-    if (!curves_fit_shared(st.D, tallies)) {  // the state of one replicate does not fit one SM's shared memory
-        if (!gslices || nslices < 1) return cudaErrorInvalidValue;
-        int nw = (nslices + num_sms - 1) / num_sms;  // spread over the SMs, at most 16 warps per CTA
-        if (nw > 16) nw = 16;
-        int grid = nslices / nw;
-        if (grid > (rep_count + nw - 1) / nw) grid = (rep_count + nw - 1) / nw;
-        curves_large_kernel<<<grid, nw * 32, 0, stream>>>(st, a, (int)curves_slice_bytes(st.D, tallies), gslices);
-        return cudaGetLastError();
-    }
-    const int slice = (int)curves_slice_bytes(st.D, tallies);
-    int nw = (227 * 1024) / slice;
-    if (nw > 16) nw = 16;
-    cudaError_t e = cudaFuncSetAttribute(curves_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, nw * slice);
-    if (e != cudaSuccess) return e;
-    int per_sm = 1;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, curves_kernel, nw * 32, (size_t)nw * slice);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    int grid = (rep_count + nw - 1) / nw;
-    if (grid > num_sms * per_sm) grid = num_sms * per_sm;
-    if (grid < 1) grid = 1;
-    curves_kernel<<<grid, nw * 32, (size_t)nw * slice, stream>>>(st, a, slice);
-    return cudaGetLastError();
+    return launch_replay(curves_kernel, curves_large_kernel, curves_slice_bytes(st.D, removed || sampled), rep_count,
+                         stream, num_sms, gslices, nslices, st, a);
+}
+
+cudaError_t launch_trajectories(const DevState &st, const double *times, int npoints, long long *out, cudaStream_t stream,
+                                int num_sms, unsigned char *gslices, int nslices) {
+    CurveArgs a = {};
+    a.rep_first = 0; a.rep_count = st.R; a.step_num = npoints - 1;
+    TrajArgs t;
+    t.times = times; t.out = out;
+    return launch_replay(trajectories_kernel, trajectories_large_kernel, trajectories_slice_bytes(st.D), st.R, stream,
+                         num_sms, gslices, nslices, st, a, t);
 }
 
 }  // namespace vg

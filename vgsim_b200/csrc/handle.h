@@ -90,6 +90,10 @@ struct Handle {
     int *arch_cnt = nullptr, *arch_need = nullptr;  // scratch of vgsim_archive_tau_log: non-zero counts per dense row / per replicate
     size_t arch_cnt_cap = 0;
     std::vector<int> rep_pp_host;  // host copy of the replicate -> parameter point map
+    // outputs of vgsim_trajectories / vgsim_lineages_through_time and the device copy of their grid: grown, never shrunk
+    double *grid_buf = nullptr;
+    long long *traj_buf = nullptr, *ltt_buf = nullptr;
+    size_t grid_cap = 0, traj_cap = 0, ltt_cap = 0;
     // event pairs that bracket the hot kernels on the handle's stream: a ring, so that a pipelined driver can read the
     // duration of launch `id` after the fact (vgsim_kernel_ms) instead of blocking on every launch
     static const int NTIMER = 64;
@@ -135,10 +139,19 @@ cudaError_t launch_direct_large(const DevState &st, const SimArgs &a, const DLLa
 // one replicate's curve slice in bytes; when it does not fit one SM's shared memory, launch_curves replays in gslices,
 // a device scratch of nslices >= 1 such slices
 size_t curves_slice_bytes(const Dims &D, bool tallies);
-bool curves_fit_shared(const Dims &D, bool tallies);
 cudaError_t launch_curves(const DevState &st, int rep_first, int rep_count, int step_num, long long *inf, long long *sus,
                           long long *removed, long long *sampled, double *time_points, int *last_point,
                           cudaStream_t stream, int num_sms, unsigned char *gslices, int nslices);
+// trajectories of every replicate on the grid times[npoints] (device), out[R][npoints][2K + 2H]; gslices as above, slices
+// of trajectories_slice_bytes
+size_t trajectories_slice_bytes(const Dims &D);
+cudaError_t launch_trajectories(const DevState &st, const double *times, int npoints, long long *out, cudaStream_t stream,
+                                int num_sms, unsigned char *gslices, int nslices);
+// lineages through time of every replicate's genealogy on the grid times[npoints] (device), out[R][npoints]
+int ltt_max_points();
+cudaError_t launch_ltt(const DevState &st, const long long *node_off, const int *parent, const double *time,
+                       const int *n_nodes, int *scratch, const double *times, int npoints, long long *out,
+                       cudaStream_t stream, int num_sms);
 cudaError_t launch_rates_tap(const DevState &st, int r, double *ev, double *hp, double *popRate, double *migPop,
                              double *totals, cudaStream_t stream);
 cudaError_t launch_rates_large(const DevState &st, const DLLayout &L, double *slice, int r, double *ev, double *hp,

@@ -5,7 +5,8 @@ The reference runs one `Simulator` per parameter point and process.  Here a swee
 parameter blobs are uploaded once (`vgsim_upload_params`), `vgsim_set_replicate_params` maps replicates to points,
 and a single launch of each kernel advances all of them; a rank owns a contiguous range of the global point list
 (`_shard.replicate_range`), replicate seeds are functions of the GLOBAL replicate id, and the only exchange is the
-all-gather of the fixed-size summaries.
+all-gather of fixed-size rows: the summaries, and where wanted the trajectories and lineages through time on a grid
+shared by every replicate (`_shard.gather_summaries` moves any of them).
 """
 import numpy as np
 
@@ -94,6 +95,15 @@ class Sweep:
     def summaries(self):
         """[points on this rank, replicates_per_point, NSUMMARY] (include/vgsim_b200.h: vgsim_summaries)."""
         return self.h.summaries().reshape(self.hi - self.lo, self.rpp, _capi.NSUMMARY)
+
+    def trajectories(self, times):
+        """Trajectories on the shared grid `times` (Handle.trajectories), each array shaped [points on this rank,
+        replicates_per_point, T, K or H]; -1 where a replicate's run ended before the grid point."""
+        return {k: v.reshape((self.hi - self.lo, self.rpp) + v.shape[1:]) for k, v in self.h.trajectories(times).items()}
+
+    def lineages_through_time(self, times):
+        """[points on this rank, replicates_per_point, T] lineages through time of every replicate's genealogy."""
+        return self.h.lineages_through_time(times).reshape(self.hi - self.lo, self.rpp, -1)
 
     def counters(self):
         return self.h.get_counters()
