@@ -124,6 +124,23 @@ int vgsim_state_dev(vgsim_handle h, void **dSx, void **dI);
  * setters does; batch drivers call it between independent batches, followed by vgsim_set_state). */
 int vgsim_reset(vgsim_handle h);
 
+/* Resampling and branching on the device: for every r with source[r] != r, replicate r's run becomes the run replicate
+ * source[r] had before the call; replicates with source[r] == r are untouched.  Copied: I, Sx and the Restart snapshot,
+ * live contact density, lockdown flags and records, effective migration, clock, rate totals, all counters, the Philox
+ * epoch, error bits, the recycled-row count, the event log rows [0, events), the (time, tau) rows [0, leaps), the dense
+ * rows not yet archived and the archive itself (used rows only, never whole capacities).  Not copied: the seed and the
+ * parameter point -- r keeps its own, and its derived rates follow its point at the next simulate call or rate tap.  A
+ * clone given its source's seed then continues exactly like the source; with its own seed it is an independent run from
+ * the same history.
+ * Rule: a replicate that is copied from keeps its own run, source[source[r]] == source[r] for every r (survivors keep
+ * their slots, extra copies fill the slots of replicates that die), so the gather needs no staging memory.  A map that
+ * breaks it, or an index outside [0, R) ("replicate out of range"), fails with a message naming r and its source, and
+ * changes nothing.  Genealogy outputs are dropped as after a simulate call.  Whatever a replicate holds is copied: after
+ * vgsim_genealogy, the rewound infectious counts.  Stream-ordered, no host synchronisation: one small copy of the map and
+ * one kernel launch on the handle's stream; the identity map enqueues nothing.  Works before the first simulate call
+ * (the configured state is copied) and on every shape vgsim_create accepts. */
+int vgsim_resample(vgsim_handle h, const int32_t *source /*[R]*/);
+
 /* Long runs in leap blocks: drop the event log / dense tau log of every replicate but keep compartments, clocks,
  * event counters, lockdown state and the Philox epoch, so that the next simulate call continues the same
  * trajectories into recycled log capacity (the reference can only grow its log, src/events.pxi:52-68; 4,096

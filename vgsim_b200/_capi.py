@@ -39,7 +39,7 @@ def _load():
         # in-tree build (nvcc cross-compiles sm_100a without a GPU); raises if nvcc is unavailable
         _build.build()
     lib = ctypes.CDLL(LIB_PATH)
-    if not hasattr(lib, "vgsim_lineages_through_time_dev") and LIB_PATH == _build.LIB and _build.have_nvcc():
+    if not hasattr(lib, "vgsim_resample") and LIB_PATH == _build.LIB and _build.have_nvcc():
         # a library built from older sources (it lacks the newest entry point): rebuild once and load the new file
         del lib
         _build.build(force=True)
@@ -94,6 +94,7 @@ def _load():
         "vgsim_trajectories_dev": (c_int, [P, P, c_int64, ctypes.POINTER(c_void_p)]),
         "vgsim_lineages_through_time": (c_int, [P, P, c_int64, P]),
         "vgsim_lineages_through_time_dev": (c_int, [P, P, c_int64, ctypes.POINTER(c_void_p)]),
+        "vgsim_resample": (c_int, [P, P]),
         "vgsim_launch_count": (c_int64, [P]),
         "vgsim_set_tau_variant": (c_int, [P, c_int]),
         "vgsim_set_direct_variant": (c_int, [P, c_int]),
@@ -271,6 +272,20 @@ class Handle:
         lock = np.empty((self.R, self.K), np.int64)
         _ck(lib.vgsim_get_state(self._h, _p(Sx), _p(I), _p(cd), _p(lock)))
         return (Sx, I, cd, lock) if full else (Sx, I)
+
+    def resample(self, source):
+        """Replicate r's whole run becomes the run replicate source[r] had before the call (include/vgsim_b200.h:
+        vgsim_resample); seeds and parameter points stay with the slot.  A replicate that is copied from must keep its
+        own run (source[source[r]] == source[r])."""
+        s = np.asarray(source)
+        if s.shape != (self.R,) or not np.issubdtype(s.dtype, np.integer):
+            raise ValueError("resample: source must be an integer array of length %d (got %s of shape %s)"
+                             % (self.R, s.dtype, s.shape))
+        bad = np.flatnonzero((s < -2 ** 31) | (s >= 2 ** 31))
+        if bad.size:
+            raise ValueError("resample: replicate %d copies from %d: replicate out of range" % (bad[0], s[bad[0]]))
+        s = np.ascontiguousarray(s, dtype=np.int32)
+        _ck(lib.vgsim_resample(self._h, _p(s)))
 
     # ---- hot path
     def simulate_direct(self, iterations, sample_size=-1, time=-1.0, attempts=200, sync=True):

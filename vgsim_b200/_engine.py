@@ -433,6 +433,20 @@ class BirthDeathModel:
         self._refresh_host_state()
         self._print_stop_reason(sample_size, time, size)
 
+    def resample(self, source):
+        """Replicate r continues the run of replicate source[r] (source: integers, one per replicate): state, counters,
+        logs and lockdown records are copied on the device, the seed and the parameter point stay with r.  A replicate
+        that is copied from keeps its own run (source[source[r]] == source[r], what `resample.systematic_map` builds).
+        The genealogy is dropped, as after a simulate call."""
+        s = np.asarray(source)
+        if s.shape != (self.replicates,) or not np.issubdtype(s.dtype, np.integer):
+            raise ValueError("resample: source must be an integer array of length %d (got %s of shape %s)"
+                             % (self.replicates, s.dtype, s.shape))
+        h = self._sync_params()
+        h.resample(s)
+        self._genealogy_done = False
+        self._refresh_host_state()
+
     def _log_rows(self):
         """events.ptr of replicate 0 before a call (0 before the first one)."""
         c = getattr(self, "_counters", None)

@@ -231,6 +231,12 @@ class Simulator:
         if self.verbose:
             self.simulation.Stats(time.time() - start_time)
 
+    def resample(self, source):
+        """Replicate r continues the run of replicate source[r], its whole history included; seeds and parameters stay
+        with r.  A replicate that is copied from keeps its own run: build maps with `vgsim_b200.resample.systematic_map`
+        (resampling by weights) or fork one replicate into all (``[s] * replicates``)."""
+        self.simulation.resample(source)
+
     def genealogy(self, seed=None):
         start_time = time.time()
         self.simulation.GetGenealogy(seed)

@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvgsim_b200.so")
-SOURCES = ["capi.cu", "tau_kernel.cu", "prep_kernels.cu", "direct_kernel.cu", "direct_large_kernel.cu", "genealogy_kernel.cu", "curves_kernel.cu", "lineages_kernel.cu", "archive_kernel.cu", "param_grid_kernel.cu", "test_taps.cu"]
+SOURCES = ["capi.cu", "tau_kernel.cu", "prep_kernels.cu", "direct_kernel.cu", "direct_large_kernel.cu", "genealogy_kernel.cu", "curves_kernel.cu", "lineages_kernel.cu", "archive_kernel.cu", "param_grid_kernel.cu", "resample_kernel.cu", "test_taps.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -505,6 +505,7 @@ static int ensure_ev_cap(Handle *h, long long need) {
     DevState &st = h->st;
     if (need <= st.ev_cap) return 0;
     long long nc = std::max(need, std::min(st.ev_cap + st.ev_cap / 2, need + (1LL << 16)));  // blocked runs: not one regrow per block
+    nc = (nc + 1) & ~1LL;  // even: every replicate's rows start 16-byte aligned for the vector copies of vgsim_resample
     if (grow2d(h, &st.ev_time, st.ev_cap, nc, h->ev_bound, 1)) return 1;
     if (grow2d(h, &st.ev_desc, st.ev_cap, nc, h->ev_bound, 1)) return 1;
     st.ev_cap = nc;
@@ -1151,6 +1152,39 @@ int vgsim_lineages_through_time(vgsim_handle h, const double *times, int64_t T, 
     if (vgsim_lineages_through_time_dev(h, times, T, nullptr)) return 1;
     CK(cudaMemcpyAsync(out, h->ltt_buf, (size_t)h->R * T * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int vgsim_resample(vgsim_handle h, const int32_t *source) {
+    CK(cudaSetDevice(h->device));
+    const int R = h->R;
+    std::vector<int2> pairs;
+    for (int r = 0; r < R; r++) {
+        const int s = source[r];
+        if (s < 0 || s >= R)
+            return fail("resample: replicate " + std::to_string(r) + " copies from " + std::to_string(s) +
+                        ": replicate out of range");
+    }
+    for (int r = 0; r < R; r++) {
+        const int s = source[r];
+        if (s == r) continue;
+        if (source[s] != s)
+            return fail("resample: replicate " + std::to_string(r) + " copies from " + std::to_string(s) +
+                        ", which copies from " + std::to_string(source[s]) +
+                        " (a replicate that is copied from must keep its own run)");
+        pairs.push_back(make_int2(r, s));
+    }
+    // genealogy outputs are dropped as after a simulate call (for the identity map as well); the host bounds are maxima
+    // over replicates and stay valid
+    h->gen.valid = false;
+    if (pairs.empty()) return 0;
+    if (ensure_buf(h, &h->resample_pairs, h->resample_cap, pairs.size())) return 1;
+    CK(cudaMemcpyAsync(h->resample_pairs, pairs.data(), pairs.size() * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
+    int n = 0;
+    cudaError_t e = launch_resample(h->st, h->resample_pairs, (int)pairs.size(), h->ev_bound, h->leap_bound, h->dense_bound,
+                                    h->stream, &n);
+    h->launches += n;
+    if (e != cudaSuccess) return fail(std::string("resample kernel: ") + cudaGetErrorString(e));
     return 0;
 }
 

@@ -94,6 +94,8 @@ struct Handle {
     double *grid_buf = nullptr;
     long long *traj_buf = nullptr, *ltt_buf = nullptr;
     size_t grid_cap = 0, traj_cap = 0, ltt_cap = 0;
+    int2 *resample_pairs = nullptr;  // (destination, source) pairs of the last vgsim_resample: grown, never shrunk
+    size_t resample_cap = 0;
     // event pairs that bracket the hot kernels on the handle's stream: a ring, so that a pipelined driver can read the
     // duration of launch `id` after the fact (vgsim_kernel_ms) instead of blocking on every launch
     static const int NTIMER = 64;
@@ -159,5 +161,9 @@ cudaError_t launch_rates_large(const DevState &st, const DLLayout &L, double *sl
 bool tau_fits(const Dims &D, int uniform_pp);
 int param_grid_slots(int num_sms, int n_points);
 cudaError_t launch_param_grid(const DevState &st, const GridArgs &g, cudaStream_t stream);
+// the gather of vgsim_resample over pairs[ndst] (device); the bounds are the handle's host maxima of log rows, leaps and
+// dense rows per replicate.  nlaunch: kernel launches enqueued (0 when ndst == 0)
+cudaError_t launch_resample(const DevState &st, const int2 *pairs, int ndst, long long ev_bound, long long leap_bound,
+                            long long dense_bound, cudaStream_t stream, int *nlaunch);
 
 }  // namespace vg

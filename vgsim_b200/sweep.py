@@ -89,6 +89,12 @@ class Sweep:
         else:
             raise ValueError("Unknown method. Choose between 'direct' and 'tau'.")
 
+    def resample(self, source):
+        """Replicate r of this rank continues the run of replicate source[r] of this rank (rank-local indices, one per
+        replicate, points in order and replicates_per_point within each); r keeps its seed and parameter point, so a
+        fork of one history maps into every point of the sweep (Handle.resample)."""
+        self.h.resample(source)
+
     def genealogy(self, seed=None):
         self.h.genealogy(seed, None)
 
